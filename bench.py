@@ -2,7 +2,7 @@
 """
 Benchmark of the PGW4ERA5 per-timestep path on B200 (contract: see DESIGN.md "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): global 0.25 degree ERA5 timesteps/s.  One "step" is one
 full ERA5 timestep (721x1440 columns x 137 levels, plev19 deltas) through the
@@ -17,7 +17,9 @@ Further legs of the same line: `e2e` (host buffers, copies inside the timing)
 with the platform's measured link bound, `roofline`, `cpu_baseline` (N = 1),
 `config.broadcast` and `config.latband` (N > 1: one global snapshot of BASELINE
 configs[4] in latitude bands).  `--impl reference`: the reference path's CPU
-implementation on all host cores.
+implementation on all host cores.  `--dump-outputs DIR`: what the last timed
+step returned, as .npy files (see `dump_outputs`); the inputs depend only on
+the arguments, so two builds can be compared output for output.
 
 Prints ONE JSON line (rank 0).
 """
@@ -37,6 +39,7 @@ sys.path.insert(0, ROOT)
 
 METRIC = "global 0.25deg ERA5 timesteps/s"
 GRIDS = {"GL": (721, 1440), "EU": (201, 281)}
+DUMP_COLUMNS = 8192
 
 
 def algorithmic_bytes(ncol, nlev=137, nplev=19, nsoil=4):
@@ -329,6 +332,34 @@ def latband_leg(a, dev, rank, world, barrier):
         settings.thresh_phi_ref_max_error = old
 
 
+def dump_outputs(out_dir, res):
+    """Write the output dict of one timestep (`Pending.result()`) to `out_dir` as .npy files: the surface fields
+    PS, T_SKIN, FR_SEA_ICE, delta_ps whole as float32 [lat, lon]; T_SO, T, QV, U, V as float32 [levels, columns]
+    at DUMP_COLUMNS columns drawn once from a fixed seed (ascending flat lat * lon indices, the same for every
+    run on the same grid); n_iter and phi_max_errors as float64.  About 40 MB on the global grid.
+    Sea ice is undefined (NaN) over land, as in the ERA5 files and the reference's output: FR_SEA_ICE_defined
+    is 1 where FR_SEA_ICE holds a value and 0 where the path returned NaN, which FR_SEA_ICE stores as 0, so
+    that every file holds finite numbers.  A NaN anywhere else is a defect and is written as it is."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    ny, nx = res["PS"].shape[-2:]
+    ncol = ny * nx
+    cols = np.sort(np.random.default_rng(0).choice(ncol, min(DUMP_COLUMNS, ncol), replace=False))
+    idx = torch.as_tensor(cols, device=res["PS"].device)
+    arrays = {name: res[name].reshape(ny, nx) for name in ("PS", "T_SKIN", "FR_SEA_ICE", "delta_ps")}
+    for name in ("T_SO", "T", "QV", "U", "V"):
+        arrays[name] = res[name].reshape(res[name].shape[1], ncol).index_select(1, idx)
+    for name, t in arrays.items():
+        a = t.cpu().numpy().astype(np.float32)
+        if name == "FR_SEA_ICE":
+            defined = ~np.isnan(a)
+            np.save(os.path.join(out_dir, "FR_SEA_ICE_defined.npy"), defined.astype(np.float32))
+            a = np.where(defined, a, np.float32(0.0))
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    np.save(os.path.join(out_dir, "n_iter.npy"), np.array([res["n_iter"]], dtype=np.float64))
+    np.save(os.path.join(out_dir, "phi_max_errors.npy"), np.array(res["phi_max_errors"], dtype=np.float64))
+
+
 def run_ours(a):
     import torch
     import torch.distributed as dist
@@ -434,6 +465,8 @@ def run_ours(a):
     barrier()
     if sampler:
         sampler.mark_stop()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, last.result())        # before the legs below reuse the output buffers
     ms = ev0.elapsed_time(ev1)
     kernel_ms = [e0.elapsed_time(e1) for e0, e1 in eng.kernel_events]
     # time the GPU spent in the column kernel per launch: the union of the launches' intervals (with several
@@ -598,7 +631,13 @@ def main():
     ap.add_argument("--streams", type=int, default=2, help="CUDA streams the timesteps alternate between")
     ap.add_argument("--no-latband", action="store_true")
     ap.add_argument("--latband-snapshots", type=int, default=100)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0) to DIR as .npy files")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     a.warmup = max(a.warmup, 3) if a.impl == "ours" else a.warmup
     if a.impl == "reference":
         run_reference(a)

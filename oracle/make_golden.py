@@ -1,14 +1,15 @@
 """
 TEST INFRASTRUCTURE ONLY -- generates tests/golden/reference_functions.npz by
-running the UNMODIFIED reference functions from /root/reference/functions.py.
+running the UNMODIFIED reference functions from the functions.py of a PGW4ERA5
+checkout (its directory in $PGW4ERA5_REFERENCE).
 
 The reference cannot be imported as-is in the build container (xarray, pyvista,
 pyproj are absent), so empty stand-in modules are inserted into ``sys.modules``
 for those three names only; every function exercised below is pure
-numpy/numba and never touches them.  /root/reference does not exist on the GPU
-box, hence the outputs are committed as a small fixture.
+numpy/numba and never touches them.  The reference is not part of this
+repository, hence the outputs are committed as a small fixture.
 
-    python oracle/make_golden.py        (run in the build container)
+    PGW4ERA5_REFERENCE=/path/to/PGW4ERA5 python oracle/make_golden.py
 """
 import os
 import sys
@@ -16,7 +17,7 @@ import types
 
 import numpy as np
 
-REF = "/root/reference"
+REF = os.environ.get("PGW4ERA5_REFERENCE", "")
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "tests", "golden",
                    "reference_functions.npz")
 
@@ -28,6 +29,8 @@ def import_reference_functions():
             for a in attrs:
                 setattr(mod, a, object)
             sys.modules[name] = mod
+    if not os.path.isfile(os.path.join(REF, "functions.py")):
+        raise SystemExit("set PGW4ERA5_REFERENCE to the directory of a PGW4ERA5 checkout")
     sys.path.insert(0, REF)
     import functions  # noqa: the reference's functions.py
     return functions

@@ -1,17 +1,18 @@
 """
 TEST INFRASTRUCTURE ONLY -- generates tests/golden/reference_glue.npz by running the UNMODIFIED
-reference code -- /root/reference/functions.py and step_03_apply_to_era.py, including the xarray-bound
+reference code -- functions.py and step_03_apply_to_era.py of the PGW4ERA5 checkout in
+$PGW4ERA5_REFERENCE, including the xarray-bound
 functions (integ_geopot, load_delta, load_delta_interp, vert_interp_delta, interp_logp_4d,
 regrid_lat_lon, filter_data and the whole of pgw_for_era5) -- on small seeded cases.
 
 xarray is absent from the build container; ``oracle/xrlite.py`` (a restatement of xarray's published
 semantics for exactly the calls the reference makes) is installed as ``sys.modules['xarray']`` for
-this script only, pyvista/pyproj are empty stand-ins (never touched on this path).  /root/reference
-does not exist on the GPU box, hence the inputs AND the reference's outputs are committed as a
-fixture; ``tests/test_oracle_glue_golden.py`` pins the oracle against it and
-``tests/test_timestep_gpu.py`` the CUDA path.
+this script only, pyvista/pyproj are empty stand-ins (never touched on this path).  The reference
+is not part of this repository, hence the inputs AND the reference's outputs are committed as a
+fixture (written by oracle/golden.py); ``tests/test_oracle_glue_golden.py`` pins the oracle against
+it and ``tests/test_timestep_gpu.py`` the CUDA path.
 
-    python oracle/make_golden_glue.py        (run in the build container)
+    PGW4ERA5_REFERENCE=/path/to/PGW4ERA5 python oracle/make_golden_glue.py
 """
 import contextlib
 import io
@@ -27,12 +28,15 @@ from scipy.io import netcdf_file
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-REF = "/root/reference"
+REF = os.environ.get("PGW4ERA5_REFERENCE", "")
 OUT = os.path.join(ROOT, "tests", "golden", "reference_glue.npz")
 sys.path.insert(0, ROOT)
+from oracle import golden  # noqa: E402
 
 
 def import_reference():
+    if not os.path.isfile(os.path.join(REF, "functions.py")):
+        raise SystemExit("set PGW4ERA5_REFERENCE to the directory of a PGW4ERA5 checkout")
     from oracle import xrlite
     sys.modules["xarray"] = xrlite
     for name, attrs in (("pyvista", ("PolyData",)), ("pyproj", ("Geod",))):
@@ -353,7 +357,7 @@ def main(out=OUT):
         g["fd_in"] = raw
         g["fd_out"] = read_nc(os.path.join(tmp, "smooth.nc"))["ta"]
 
-    np.savez_compressed(out, **g)
+    golden.save(out, g)
     print("wrote", out, len(g), "arrays", os.path.getsize(out), "bytes")
 
 

@@ -85,4 +85,4 @@ def main(ref_dir):
 
 
 if __name__ == "__main__":
-    main(sys.argv[1] if len(sys.argv) > 1 else "/root/reference")
+    main(sys.argv[1] if len(sys.argv) > 1 else os.environ.get("PGW4ERA5_REFERENCE", "."))

@@ -4,6 +4,7 @@ import numpy as np
 import pytest
 
 from oracle import pgw_oracle as O
+from oracle.golden import load as load_golden
 
 pytestmark = pytest.mark.gpu
 
@@ -111,7 +112,7 @@ def test_integ_geopot_vs_oracle(F):
 def test_integ_geopot_vs_executed_reference(F):
     """functions.py:128-189 run unmodified over oracle/xrlite.py (tests/golden/reference_glue.npz)."""
     import os
-    G = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_glue.npz"))
+    G = load_golden(os.path.join(os.path.dirname(__file__), "golden", "reference_glue.npz"))
     ak, bk, ps = G["ig_ak"], G["ig_bk"], G["ig_ps"]
     pa_hl = ak[None, :, None, None] + ps[:, None] * bk[None, :, None, None]
     for tag, p_ref in (("30000", 30000), ("50000", 50000.0), ("col", G["ig_pref_col"])):

@@ -1,7 +1,7 @@
 """
 The oracle against the UNMODIFIED reference executed in the build container, including its
 xarray-bound functions and the whole of ``pgw_for_era5`` (tests/golden/reference_glue.npz, written by
-oracle/make_golden_glue.py: /root/reference/functions.py and step_03_apply_to_era.py run over
+oracle/make_golden_glue.py: the reference's functions.py and step_03_apply_to_era.py run over
 oracle/xrlite.py, a restatement of the xarray semantics they rely on).  Tolerances are float64
 round-off unless a comment says what else is in them.
 """
@@ -12,8 +12,9 @@ import numpy as np
 import pytest
 
 from oracle import pgw_oracle as O
+from oracle.golden import load as load_golden
 
-G = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_glue.npz"))
+G = load_golden(os.path.join(os.path.dirname(__file__), "golden", "reference_glue.npz"))
 
 
 def md(a, b):
@@ -25,10 +26,10 @@ def md(a, b):
 
 def golden_case():
     """The inputs of the per-timestep goldens (5 x 6 columns, 137 levels, plev19 monthly deltas)."""
-    era = {k[len("case_era_"):]: G[k] for k in G.files if k.startswith("case_era_")}
+    era = {k[len("case_era_"):]: G[k] for k in G if k.startswith("case_era_")}
     times = G["case_delta_time"].astype("datetime64[ns]")
     deltas = {}
-    for k in G.files:
+    for k in G:
         if k.startswith("case_delta_") and k not in ("case_delta_time", "case_delta_plev"):
             d = G[k]
             deltas[k[len("case_delta_"):]] = dict(time=times, data=d, plev=G["case_delta_plev"] if d.ndim == 4 else None)

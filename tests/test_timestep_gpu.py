@@ -320,16 +320,17 @@ def test_polynomial_fixed_point_large_ps_change_falls_back():
 def _golden_case():
     import os
     from datetime import datetime
-    G = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_glue.npz"))
+    from oracle.golden import load as load_golden
+    G = load_golden(os.path.join(os.path.dirname(__file__), "golden", "reference_glue.npz"))
     era = {}
-    for k in G.files:
+    for k in G:
         if k.startswith("case_era_"):
             v = G[k]
             era[k[len("case_era_"):]] = torch.from_numpy(v) if v.dtype == np.float32 else v
     era["akm"], era["bkm"] = 0.5 * (era["ak"][1:] + era["ak"][:-1]), 0.5 * (era["bk"][1:] + era["bk"][:-1])
     times = G["case_delta_time"].astype("datetime64[ns]")
     deltas = {}
-    for k in G.files:
+    for k in G:
         if k.startswith("case_delta_") and k not in ("case_delta_time", "case_delta_plev"):
             d = G[k]
             deltas[k[len("case_delta_"):]] = dict(time=times, data=torch.from_numpy(d),
