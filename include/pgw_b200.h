@@ -365,7 +365,8 @@ int pgw_ps_adjust_f64(const double *phi_pgw, const double *phi_era, const double
  *   j0,j1 [ny_t] source rows (-1 = south-pole row, -2 = north-pole row,
  *                i.e. the zonal mean of row 0 / ny_s-1), wy [ny_t] weight of j1
  *   i0,i1 [nx_t] source columns (already wrapped), wx [nx_t] weight of i1
- *   polemean [nfield, 2] zonal means (filled by pgw_zonal_mean_f32)
+ *   polemean [nfield, 2] zonal means (filled by pgw_zonal_mean_f32: the mean of
+ *                the valid points of the row, skipping NaN like xarray; NaN if none)
  * pgw_smooth_harmonic_f32 replaces filter_data()/harmonic_ac_analysis(),
  * functions.py:606-740: per grid point mean + 3 harmonics of the nt-long series.
  * ---------------------------------------------------------------------- */

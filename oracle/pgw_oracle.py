@@ -497,6 +497,14 @@ def _interp1d_axis(x, y, x_new, axis):
     return np.moveaxis(y_new, 0, axis)
 
 
+def _nanmean_lastaxis(x):
+    """xarray's DataArray.mean(dim=...) on float data (skipna): the mean of the valid points, NaN if none."""
+    import warnings
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore", RuntimeWarning)       # "Mean of empty slice" for an all-NaN row
+        return np.nanmean(x, axis=-1, keepdims=True)
+
+
 def regrid_lat_lon(data, lat_gcm, lon_gcm, targ_lat, targ_lon):
     """
     functions.py:748-898 (xarray-only branch).  data [..., nlat_gcm, nlon_gcm]
@@ -513,14 +521,13 @@ def regrid_lat_lon(data, lat_gcm, lon_gcm, targ_lat, targ_lon):
     if lat[0] > lat[-1]:                                     # :822-829
         lat = lat[::-1]
         data = data[..., ::-1, :]
+    # the pole rows are xarray means over lon, which skip NaN (all-NaN row -> NaN)
     if np.max(targ_lat) + dlat_gcm > 89.9:                   # :833-837
-        north = np.broadcast_to(data[..., -1:, :].mean(axis=-1, keepdims=True),
-                                data[..., -1:, :].shape)
+        north = np.broadcast_to(_nanmean_lastaxis(data[..., -1:, :]), data[..., -1:, :].shape)
         data = np.concatenate([data, north], axis=-2)
         lat = np.concatenate([lat, [90.0]])
     if np.min(targ_lat) - dlat_gcm < -89.9:                  # :838-842
-        south = np.broadcast_to(data[..., :1, :].mean(axis=-1, keepdims=True),
-                                data[..., :1, :].shape)
+        south = np.broadcast_to(_nanmean_lastaxis(data[..., :1, :]), data[..., :1, :].shape)
         data = np.concatenate([south, data], axis=-2)
         lat = np.concatenate([[-90.0], lat])
     if (np.max(targ_lat) > np.max(lat)) or (np.min(targ_lat) < np.min(lat)):  # :845-856

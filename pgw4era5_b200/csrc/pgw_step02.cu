@@ -16,7 +16,9 @@ int pgw_ensure_smem(const void *kernel, int slot, size_t smem, int np);
 namespace pgw {
 
 // zonal mean of the first and last source row of every field: the values the
-// reference puts on the synthetic pole rows (functions.py:833-842)
+// reference puts on the synthetic pole rows (functions.py:833-842).  The reference
+// takes it with xarray's DataArray.mean, which skips NaN for float data: the mean of
+// the valid points of the row, NaN only when the whole row is missing.
 __global__ void __launch_bounds__(128)
 zonal_mean_kernel(const float *__restrict__ src, float *__restrict__ polemean, long long nfield, int ny_s,
                   int nx_s) {
@@ -24,16 +26,25 @@ zonal_mean_kernel(const float *__restrict__ src, float *__restrict__ polemean, l
     const int which = blockIdx.y;                   // 0: row 0, 1: row ny_s-1
     const float *row = src + (f * ny_s + (which ? ny_s - 1 : 0)) * (long long)nx_s;
     double s = 0.0;
-    for (int i = threadIdx.x; i < nx_s; i += blockDim.x) s += (double)row[i];
+    int n = 0;
+    for (int i = threadIdx.x; i < nx_s; i += blockDim.x) {
+        const float v = row[i];
+        if (!isnan(v)) { s += (double)v; ++n; }
+    }
     __shared__ double part[4];
+    __shared__ int cnt[4];
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-    if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = s;
+    for (int o = 16; o > 0; o >>= 1) {
+        s += __shfl_xor_sync(0xffffffffu, s, o);
+        n += __shfl_xor_sync(0xffffffffu, n, o);
+    }
+    if ((threadIdx.x & 31) == 0) { part[threadIdx.x >> 5] = s; cnt[threadIdx.x >> 5] = n; }
     __syncthreads();
     if (threadIdx.x == 0) {
         double t = 0.0;
-        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) t += part[w];
-        polemean[f * 2 + which] = (float)(t / (double)nx_s);
+        int c = 0;
+        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) { t += part[w]; c += cnt[w]; }
+        polemean[f * 2 + which] = c ? (float)(t / (double)c) : NAN;
     }
 }
 

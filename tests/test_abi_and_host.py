@@ -2,6 +2,7 @@
 host logic (calendar brackets, regrid tables, partitioning, NetCDF shim) against the oracle."""
 import os
 import re
+import warnings
 from datetime import datetime
 
 import numpy as np
@@ -81,8 +82,11 @@ def test_leap_day_dropped_from_daily_series():
 
 
 def _emulate_gather(data, tb):
-    pm0 = data[..., 0, :].mean(-1, dtype=np.float64).astype(np.float32).astype(np.float64)
-    pm1 = data[..., -1, :].mean(-1, dtype=np.float64).astype(np.float32).astype(np.float64)
+    # zonal_mean_kernel: mean of the valid points of the first / last row (NaN if none), rounded to float32
+    with np.errstate(all="ignore"), warnings.catch_warnings():
+        warnings.simplefilter("ignore", RuntimeWarning)
+        pm0 = np.nanmean(data[..., 0, :], -1, dtype=np.float64).astype(np.float32).astype(np.float64)
+        pm1 = np.nanmean(data[..., -1, :], -1, dtype=np.float64).astype(np.float32).astype(np.float64)
 
     def at(j, i):
         out = np.empty(data.shape[:-2] + (len(j), len(i)))
@@ -121,6 +125,34 @@ def test_regrid_tables_match_oracle(case):
     got = _emulate_gather(data.astype(np.float64), F.regrid_tables(lat, lon, tlat, tlon))
     assert not np.isnan(ref).any()
     np.testing.assert_allclose(got, ref, rtol=0, atol=2e-7)
+
+
+def test_regrid_pole_rows_skip_nan():
+    """The pole rows are `north[var].mean(dim=[lon])` (functions.py:833-842): an xarray mean, which skips NaN
+    for float data.  A partly missing first / last source row gives the mean of its valid points, so the target
+    rows between the pole and that row stay finite wherever the row is; an all-NaN row gives NaN."""
+    from oracle import pgw_oracle as O
+    from oracle import xrlite as xr
+    from pgw4era5_b200 import functions as F
+    lat, lon = np.linspace(-85, 85, 18), np.arange(0.0, 360, 10.0)
+    tlat, tlon = np.linspace(-90, 90, 73), np.arange(0, 360, 7.5)
+    rng = np.random.default_rng(4)
+    data = rng.normal(size=(3, len(lat), len(lon))).astype(np.float32)
+    data[0, 0, 5:9] = np.nan                       # partly missing southernmost row
+    data[1, -1, ::9] = np.nan                      # partly missing northernmost row
+    data[2, 0, :] = np.nan                         # whole southernmost row missing
+    ref = O.regrid_lat_lon(data, lat, lon, tlat, tlon)
+    got = _emulate_gather(data.astype(np.float64), F.regrid_tables(lat, lon, tlat, tlon))
+    np.testing.assert_array_equal(np.isnan(got), np.isnan(ref))
+    np.testing.assert_allclose(got, ref, rtol=0, atol=2e-7, equal_nan=True)
+    # target rows -87.5 and 87.5 lie between a pole row and the partly missing source row: finite where that row is
+    assert 0 < np.isnan(ref[0, 1]).sum() < len(tlon) // 2 and 0 < np.isnan(ref[1, -2]).sum() < len(tlon) // 2
+    # an all-NaN row: NaN up to the next source row (-75, bracketed with row 0), finite from there on
+    assert np.isnan(ref[2, :7]).all() and np.isfinite(ref[2, 7:]).all()
+    # the pole value itself is xrlite's DataArray.mean over lon (xarray semantics restated)
+    da = xr.DataArray(data[0, :1].astype(np.float64), dims=("lat", "lon"), coords={"lat": lat[:1], "lon": lon})
+    pole = float(da.mean(dim=["lon"]).values[0])
+    assert np.isfinite(pole) and abs(ref[0, 0, 0] - pole) < 1e-12
 
 
 def test_regrid_bounds_errors():
