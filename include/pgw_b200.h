@@ -27,8 +27,9 @@
 extern "C" {
 #endif
 
-#define PGW_B200_ABI_VERSION 6   /* 6: + pgw_timestep_status, pgw_timestep_run/_finish, PGW_FLAG_REF_DTYPES, first_k,
-                                       pgw_band_pack/_unpack, pgw_band_exchange, pgw_regrid_bilinear_band_f32 */
+#define PGW_B200_ABI_VERSION 7   /* 6: + pgw_timestep_status, pgw_timestep_run/_finish, PGW_FLAG_REF_DTYPES, first_k,
+                                       pgw_band_pack/_unpack, pgw_band_exchange, pgw_regrid_bilinear_band_f32
+                                    7: + PGW_FLAG_LOCAL_PREF and its args, PGW_ERR_PREF_FLOOR, first_k[4] */
 
 /* host-side return codes */
 #define PGW_OK               0
@@ -47,6 +48,9 @@ extern "C" {
 #define PGW_ERR_PS_BOUND            (1u << 7)  /* ps left the range the column
                                                   stash was sized for: rerun
                                                   with a larger ps_bound */
+#define PGW_ERR_PREF_FLOOR          (1u << 9)  /* PGW_FLAG_LOCAL_PREF: p_ref left the range the
+                                                  column stash was sized for: rerun
+                                                  with a lower p_floor */
 
 /* extrapolation modes of interp_extrap_1d, functions.py:516-520 */
 #define PGW_EXTRAP_OFF       0
@@ -64,6 +68,12 @@ extern "C" {
                                 :147-152), -adj_factor*ps_pgw is a float32 product (step_03:302-303).  Implies
                                 PGW_FLAG_DIRECT.  Without the flag the accumulation is float64, i.e. the reference
                                 on a file that stores PS and FIS as double. */
+#define PGW_FLAG_LOCAL_PREF 4 /* p_ref_inp = None (step_03_apply_to_era.py:219-251): the reference pressure is picked
+                                per column and iteration among zg's pressure levels (determine_p_ref,
+                                functions.py:583-598) and the climate term is the zg delta on that level.  Takes the
+                                cp.async flavour; not combinable with PGW_FLAG_REF_DTYPES.  Reads the last block of
+                                pgw_timestep_args (zg .. p_ref_out); p_ref and zg_ref are ignored, p_floor sizes the
+                                column stash in place of p_ref. */
 
 #define PGW_MAX_SOIL   16
 #define PGW_MAX_ITER   64
@@ -184,7 +194,7 @@ int pgw_time_mean_f32(const float *series, int ntime, float *out, long long n, v
 /* ------------------------------------------------------------------------
  * The fused per-timestep pass.
  * Replaces the body of pgw_for_era5(), step_03_apply_to_era.py:60-343 with
- * i_reinterp = 0 and a scalar p_ref: pressures (:64-88), RELHUM (:91-94),
+ * i_reinterp = 0 and a scalar or (PGW_FLAG_LOCAL_PREF) per-column p_ref: pressures (:64-88), RELHUM (:91-94),
  * sea-ice/skin/soil update (:103-146, integrate_tos), load_delta's time blend
  * (functions.py:288-292), replace_delta_sfc + vert_interp_delta
  * (functions.py:343-431) for ta,hur,ua,va, delta application (:158-173) and
@@ -256,12 +266,26 @@ typedef struct pgw_timestep_args {
     uint64_t *maxerr;       /* [PGW_MAX_ITER] float64 bits, zeroed by the call */
     float *stats;           /* [2]: min target p, min source p (ta/hur)        */
     uint32_t *err;          /* sticky error word                               */
-    int32_t *first_k;       /* [2] or NULL: first iteration (0-based) in which PGW_ERR_PREF_BELOW_SFC /
-                               PGW_ERR_PS_BOUND fired (atomicMin; INT32_MAX = never).  The kernel runs k_spec
+    int32_t *first_k;       /* [4] or NULL: first iteration (0-based) in which PGW_ERR_PREF_BELOW_SFC /
+                               PGW_ERR_PS_BOUND / PGW_ERR_NO_PREF / PGW_ERR_PREF_FLOOR fired (atomicMin;
+                               INT32_MAX = never).  The kernel runs k_spec
                                iterations for every column, the reference stops after N: a condition that only
                                fires in an iteration >= N never happened in the reference. */
     uint32_t *poly_fallback; /* or NULL: number of (warp, iteration) pairs of the TMA flavour that left the range
                                of the dps polynomial and integrated all parked levels directly (diagnostic) */
+    /* PGW_FLAG_LOCAL_PREF only (may be zero otherwise).  p_ref_k of iteration k is the first level of zg_plev, in
+       file order, with 0.95*PS > p and 0.95*(PS + dps_k) > p, and from the second iteration on at most p_ref_{k-1}.
+       The stash covers every layer that can contain a pressure >= p_floor for ps <= ps_bound; a column whose
+       p_ref_k falls below p_floor sets PGW_ERR_PREF_FLOOR (rerun with a lower p_floor).  No qualifying level:
+       PGW_ERR_NO_PREF and p_ref NaN. */
+    pgw_tslab zg;               /* zg delta on all of zg's levels, [nzg, ncol] per time slab */
+    const double *zg_plev;      /* [nzg] DEVICE, zg's pressure levels in FILE order (distinct values) */
+    const double *zg_plev_host; /* [nzg] HOST copy (sizes the table of candidate levels) */
+    int nzg;                    /* 1..64 */
+    int reserved1;
+    double p_floor;             /* lowest p_ref the column stash is sized for */
+    uint8_t *pref_traj;         /* [k_spec, ncol] workspace: index of p_ref_k in zg_plev (255 = none) */
+    double *p_ref_out;          /* [ncol] p_ref of the iteration the result is for (finalize rewrites it for N) */
 } pgw_timestep_args;
 
 /* bytes of dynamic shared memory the column kernel needs for these args, or
@@ -269,7 +293,8 @@ typedef struct pgw_timestep_args {
 long long pgw_sizeof_timestep_args(void);   /* for FFI layout checks */
 long long pgw_timestep_smem_bytes(const pgw_timestep_args *a);
 /* 1 if pgw_timestep() takes the TMA flavour of the column kernel for these args, 0 if the
- * per-thread cp.async flavour (odd ncol, unaligned fields, PGW_COLUMN_PATH=generic) */
+ * per-thread cp.async flavour (odd ncol, unaligned fields, PGW_COLUMN_PATH=generic, PGW_FLAG_DIRECT,
+ * PGW_FLAG_REF_DTYPES, and PGW_FLAG_LOCAL_PREF on every grid: the TMA flavour handles a scalar p_ref only) */
 int pgw_timestep_uses_tma(const pgw_timestep_args *a);
 int pgw_timestep(const pgw_timestep_args *a, void *stream);
 
@@ -291,7 +316,7 @@ typedef struct pgw_timestep_status {
     pgw_timestep_result result;     /* written by finalize                                         */
     float stats[2];                 /* min target pressure, min source pressure (functions.py:417) */
     uint32_t err;                   /* PGW_ERR_* bits                                              */
-    int32_t first_k[2];             /* see pgw_timestep_args.first_k                               */
+    int32_t first_k[4];             /* see pgw_timestep_args.first_k                               */
     uint32_t poly_fallback;         /* see pgw_timestep_args.poly_fallback                         */
 } pgw_timestep_status;
 long long pgw_sizeof_timestep_status(void);
@@ -306,9 +331,9 @@ int pgw_timestep_run(const pgw_timestep_args *a, pgw_timestep_status *status_dev
 int pgw_timestep_finish(const pgw_timestep_args *a, pgw_timestep_status *status_dev,
                         pgw_timestep_status *status_host, void *stream);
 /* The status block as PGW_BAND_WORDS float64 such that an element-wise MAX over the latitude bands merges it:
- * maxerr[64] | -stats[2] | one word per error bit [32] | -first_k[2]; and back.  The stopping rule of the
+ * maxerr[64] | -stats[2] | one word per error bit [32] | -first_k[4]; and back.  The stopping rule of the
  * reference is field-global (step_03_apply_to_era.py:189,308), so this is the one exchange of band mode. */
-#define PGW_BAND_WORDS (PGW_MAX_ITER + 2 + 32 + 2)
+#define PGW_BAND_WORDS (PGW_MAX_ITER + 2 + 32 + 4)
 int pgw_band_pack(const pgw_timestep_status *status_dev, double *words_dev, void *stream);
 int pgw_band_unpack(const double *words_dev, pgw_timestep_status *status_dev, void *stream);
 /* The same exchange WITHOUT a collective library, as one kernel over peer memory (NVLink / NVSwitch): every rank owns
@@ -328,8 +353,8 @@ int pgw_band_exchange(pgw_timestep_status *status_dev, double *const *inbox_ptrs
 /* ------------------------------------------------------------------------
  * The staged per-timestep path: pgw_for_era5() run stage by stage on float64
  * device arrays with the operators above plus the small ones below.  It covers
- * the settings the fused pass does not, i_reinterp = 1
- * (step_03_apply_to_era.py:202-216, :330-343) and p_ref_inp = None (:219-251);
+ * i_reinterp = 1 (step_03_apply_to_era.py:202-216, :330-343), which the fused pass does not, and
+ * p_ref_inp = None (:219-251), the reference the fused pass's PGW_FLAG_LOCAL_PREF is tested against;
  * host orchestration: pgw4era5_b200/staged.py.
  *   pgw_surface_update        sea ice / skin / soil block, step_03:103-146
  *                             (reads only the 2-D members of the args)

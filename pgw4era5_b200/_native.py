@@ -26,12 +26,14 @@ ERR_PREF_BELOW_SFC = 1 << 5
 ERR_NO_PREF = 1 << 6
 ERR_PS_BOUND = 1 << 7
 ERR_BAND_TIMEOUT = 1 << 8
-BAND_SLOT = 64 + 2 + 32 + 2 + 4
+ERR_PREF_FLOOR = 1 << 9
+BAND_SLOT = 64 + 2 + 32 + 4 + 4
 BAND_PARITIES = 8
 FLAG_DIRECT = 1
 FLAG_REF_DTYPES = 2
+FLAG_LOCAL_PREF = 4
 RUN_NO_FINALIZE = 1
-BAND_WORDS = 64 + 2 + 32 + 2
+BAND_WORDS = 64 + 2 + 32 + 4
 INT32_MAX = 2 ** 31 - 1
 
 EXTRAP_MODES = {"off": 0, "linear": 1, "constant": 2, "nan": 3}
@@ -55,6 +57,8 @@ class TimestepArgs(C.Structure):
            ("thresh_phi_ref_max_error", C.c_double), ("k_spec", C.c_int), ("ps_bound", C.c_double)]
         + [(n, c_fp) for n in ("PS_out", "T_SKIN_out", "FR_SEA_ICE_out", "T_SO_out", "T_out", "QV_out",
                                "U_out", "V_out", "dps_out", "dps_traj", "maxerr", "stats", "err", "first_k", "poly_fallback")]
+        + [("zg", TSlab), ("zg_plev", c_fp), ("zg_plev_host", c_fp), ("nzg", C.c_int), ("reserved1", C.c_int),
+           ("p_floor", C.c_double), ("pref_traj", c_fp), ("p_ref_out", c_fp)]
     )
 
 
@@ -65,10 +69,10 @@ class TimestepResult(C.Structure):
 class TimestepStatus(C.Structure):
     """pgw_timestep_status: the device block the kernels report into and its pinned host copy."""
     _fields_ = [("maxerr", C.c_uint64 * PGW_MAX_ITER), ("result", TimestepResult), ("stats", C.c_float * 2),
-                ("err", C.c_uint32), ("first_k", C.c_int32 * 2), ("poly_fallback", C.c_uint32)]
+                ("err", C.c_uint32), ("first_k", C.c_int32 * 4), ("poly_fallback", C.c_uint32)]
 
 
-ABI_VERSION = 6          # PGW_B200_ABI_VERSION of include/pgw_b200.h
+ABI_VERSION = 7          # PGW_B200_ABI_VERSION of include/pgw_b200.h
 
 
 class NativeError(RuntimeError):

@@ -293,6 +293,8 @@ struct pgw_column_plan {
     int lst, np;        // top level of the stash, number of parked levels
     size_t smem;
     bool fast;          // ln_ratio series valid for every layer the iteration can touch
+    bool local;         // PGW_FLAG_LOCAL_PREF
+    int ncand;          // PGW_FLAG_LOCAL_PREF: zg levels >= p_floor (candidate p_ref levels)
 };
 // pgw_column_tma.cu
 bool pgw_tma_eligible(const pgw_timestep_args *a, int lst_generic, int *lst_tma, size_t *smem);

@@ -44,9 +44,13 @@ constexpr int kRing = 5;     // levels in flight per thread (cp.async ring, +1 s
 // REF: the dtypes the reference computes in on a file with float32 PS and FIS (PGW_FLAG_REF_DTYPES): float32
 // delta_ps / ps_pgw, the half-level geopotential as a float32 running sum that is rounded on every level, for the
 // ERA state and for the PGW state of every iteration, pressures as the two rounded operations ak + ps*bk.
-template <int NT, bool FAST, bool REF>
+// LOCAL: PGW_FLAG_LOCAL_PREF, p_ref per column and iteration among zg's levels (step_03:219-251).  Phase 1
+// records the ERA-state sums at every candidate level (the `ncand` zg levels >= p_floor) the column's p_ref can
+// move up to; phase 2 re-picks p_ref in every iteration and integrates the parked levels up to it.
+template <int NT, bool FAST, bool REF, bool LOCAL = false>
 __global__ void __launch_bounds__(NT, REF ? 2 : 3)
-pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, const int np) {
+pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, const int np, const int ncand) {
+    static_assert(!(REF && LOCAL), "PGW_FLAG_LOCAL_PREF runs with float64 accumulation only");
     extern __shared__ __align__(16) unsigned char smem[];
     const int L = a.nlev, K = a.nplev;
     // ---- shared memory carve-up
@@ -58,6 +62,12 @@ pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, co
     float *s_inv_plev = s_plev + K;                                     // [K]
     float *s_inv_w = s_inv_plev + K;                                    // [K] 1/log2(p[j+1]/p[j])
     float *st_r = s_inv_w + K;                                          // REF: [np][NT] (T_era + dta) - fp32 T_pgw
+    // LOCAL: zg's levels in file order, the candidates by descending pressure, per candidate and column
+    // (phi_era - FIS, residual sum) at that pressure, and the candidate slot of each zg level (-1: below p_floor)
+    double *s_zgp = reinterpret_cast<double *>((reinterpret_cast<uintptr_t>(st_r) + 15) & ~uintptr_t(15));  // [nzg]
+    double *s_cp = s_zgp + a.nzg;                                                                            // [ncand]
+    double2 *st_c = reinterpret_cast<double2 *>((reinterpret_cast<uintptr_t>(s_cp + ncand) + 15) & ~uintptr_t(15));
+    int *s_slot = reinterpret_cast<int *>(st_c + (size_t)ncand * NT);                                       // [nzg]
 
     const int tid = threadIdx.x;
     for (int i = tid; i <= L; i += NT) s_hl[i] = make_double2(a.ak[i], a.bk[i]);
@@ -71,6 +81,19 @@ pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, co
             const float p1 = (float)a.plev[a.plev_descending ? (K - 2 - i) : (i + 1)];
             s_inv_w[i] = 1.0f / log2f(p1 / p0);
         } else s_inv_w[i] = 0.0f;
+    }
+    if constexpr (LOCAL) {
+        for (int i = tid; i < a.nzg; i += NT) {
+            const double p = a.zg_plev[i];
+            int r = -1;
+            if (p >= a.p_floor) {
+                r = 0;
+                for (int j = 0; j < a.nzg; ++j) r += (a.zg_plev[j] >= a.p_floor && a.zg_plev[j] > p);
+                s_cp[r] = p;
+            }
+            s_zgp[i] = p;
+            s_slot[i] = r;
+        }
     }
     __syncthreads();
 
@@ -111,7 +134,8 @@ pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, co
     const float ps_f = __ldg(a.PS + c);
     const Pair2 r_sic = load_pair(a.siconc, c), r_ts = load_pair(a.ts, c), r_tos = load_pair(a.tos, c);
     const Pair2 r_psh = load_pair(a.ps_hist, c), r_tas = load_pair(a.tas, c), r_hurs = load_pair(a.hurs, c);
-    const Pair2 r_zg = load_pair(a.zg_ref, c);
+    Pair2 r_zg{0.0f, 0.0f};
+    if constexpr (!LOCAL) r_zg = load_pair(a.zg_ref, c);
     const float r_ice = __ldg(a.FR_SEA_ICE + c), r_land = __ldg(a.FR_LAND + c), r_skin = __ldg(a.T_SKIN + c);
     const float r_clim = __ldg(a.ts_clim + c), r_fis = __ldg(a.FIS + c);
     const double PSd = (double)ps_f;
@@ -235,12 +259,29 @@ pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, co
     LnConst lk{2.0 / 3.0, 2.0 / 5.0, 2.0 / 7.0};
     asm volatile("" : "+d"(lk.c3), "+d"(lk.c5), "+d"(lk.c7));     // keep the constants in registers
 
-    const double pref = a.p_ref;
+    double pref = a.p_ref;
+    // LOCAL: jsel = index in zg_plev of p_ref_k (-1: none); cj = next candidate slot phase 1 records
+    int jsel = -1, cj = 0;
+    int k_nopref = INT32_MAX, k_floor = INT32_MAX;
+    const double pe = 0.95 * PSd;                   // determine_p_ref's p_min_era (step_03:221-226)
+    if constexpr (LOCAL) {
+        for (int i = 0; i < a.nzg; ++i)
+            if (pe > s_zgp[i]) { jsel = i; break; }   // first iteration: ps_pgw == PS, both tests agree
+        if (jsel < 0) {
+            errbits |= PGW_ERR_NO_PREF; k_nopref = 0; pref = NAN; cj = ncand;
+        } else {
+            pref = s_zgp[jsel];
+            cj = s_slot[jsel];
+            if (cj < 0) { errbits |= PGW_ERR_PREF_FLOOR; k_floor = 0; cj = ncand; }
+        }
+        a.pref_traj[c] = (uint8_t)(jsel < 0 ? 255 : jsel);
+    }
+    const int cj0 = cj;                             // LOCAL: slot of p_ref_1
     const double2 hl_sfc = s_hl[L];
     double pb_era = fma(PSd, hl_sfc.y, hl_sfc.x);
     double acc_era = 0.0;
     bool era_open = pb_era >= pref;                 // still below p_ref
-    if (!era_open) { errbits |= PGW_ERR_PREF_BELOW_SFC; k_pref = 0; }
+    if (!era_open && !(LOCAL && jsel < 0)) { errbits |= PGW_ERR_PREF_BELOW_SFC; k_pref = 0; }
     float psn_f = ps_f;                             // ps used for QV; replaced after the iteration
     // REF: ak + ps*bk as numpy evaluates it (two rounded operations, step_03:64-66, :196-199)
     auto hyb = [](double ps, double2 h) { return __dadd_rn(h.x, __dmul_rn(ps, h.y)); };
@@ -297,6 +338,28 @@ pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, co
                         pb_era = Pt;
                     }
                 }
+                return;
+            }
+            if constexpr (LOCAL) {
+                // integ_geopot (functions.py:141-179) of the ERA state and of the residual, evaluated at every
+                // candidate level inside this layer; the PGW sum of the first iteration stops at p_ref_1
+                const double2 hl = s_hl[l];
+                const double pt = fma(PSd, hl.y, hl.x);
+                const double td = (double)t, tpd = (double)t_pgw;
+                const double rtv = rd_tv(t, q);
+                const float g = fast_rcp(fmaf(-0.378f, e_pgw, p));
+                const double tvp = fma(tpd, (double)((0.61f * 0.622f) * e_pgw * g), tpd);
+                const double res = (td + (double)dta) - tpd;
+                for (; cj < ncand && s_cp[cj] > pt; ++cj) {
+                    const double dl = ln_ratio<FAST>(pb_era, s_cp[cj], lk);
+                    st_c[(size_t)cj * NT + tid] = make_double2(fma(rtv, dl, acc_era), fma(res, dl, acc_res));
+                    if (cj == cj0) acc_pgw0 = fma(tvp, dl, acc_pgw0);
+                }
+                const double dl = ln_ratio<FAST>(pb_era, pt, lk);
+                acc_era = fma(rtv, dl, acc_era);
+                acc_res = fma(res, dl, acc_res);
+                if (cj == cj0) acc_pgw0 = fma(tvp, dl, acc_pgw0);
+                pb_era = pt;
                 return;
             }
             if (era_open) {
@@ -358,8 +421,25 @@ pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, co
         }
     }
     const double fis = (double)r_fis;
-    const double phi_era = REF ? phi_ref_era : fis + acc_era;        // acc_era holds Rd * Tv * dlnp
-    const double gdzg = blend_f64(a.zg_ref, r_zg) * kG;              // step_03:292-295
+    double phi_era = REF ? phi_ref_era : fis + acc_era;              // acc_era holds Rd * Tv * dlnp
+    double gdzg = blend_f64(a.zg_ref, r_zg) * kG;                    // step_03:292-295
+    // LOCAL: phi_era, the residual sum and the climate term (the zg delta of both time slabs, blended) at zg
+    // level j; a level below p_floor is outside the stash: flagged, the values are left as they are
+    auto take_level = [&](int j, int k) {
+        const int s = s_slot[j];
+        if (s < 0) {
+            errbits |= PGW_ERR_PREF_FLOOR; k_floor = min(k_floor, k);
+        } else {
+            const double2 v = st_c[(size_t)s * NT + tid];
+            phi_era = fis + v.x;
+            acc_res = v.y;
+        }
+        gdzg = blend_f64(a.zg, load_pair(a.zg, (uint32_t)j * n + c)) * kG;
+    };
+    if constexpr (LOCAL) {
+        if (jsel >= 0) take_level(jsel, 0);
+        else phi_era = NAN;
+    }
     const float2 *const bTe = st_Te + (size_t)(L - 1 - lst) * NT + tid;  // lowest level of the stash
     const double t_low = t_low_d;                                 // ta_pgw on the lowest level
 
@@ -383,6 +463,26 @@ pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, co
         }
         *traj = (float)dps;
         if (psn > a.ps_bound) { errbits |= PGW_ERR_PS_BOUND; k_bound = min(k_bound, k); }
+        if constexpr (LOCAL) {
+            if (k > 0) {
+                // determine_p_ref (functions.py:583-598): the first zg level, in file order, below 0.95 PS and
+                // 0.95 ps_pgw, at most the previous choice (min(p, p_ref_last) ignores a NaN p_ref_last)
+                const double pp = 0.95 * psn;
+                int j = -1;
+                for (int i = 0; i < a.nzg; ++i) {
+                    const double p = s_zgp[i];
+                    if (pe > p && pp > p) { j = i; break; }
+                }
+                if (j < 0) { errbits |= PGW_ERR_NO_PREF; k_nopref = min(k_nopref, k); }
+                else if (jsel >= 0 && !(s_zgp[j] < pref)) j = jsel;
+                if (j != jsel) {
+                    jsel = j;
+                    if (j < 0) { pref = NAN; phi_era = NAN; }
+                    else { pref = s_zgp[j]; take_level(j, k); }
+                }
+                a.pref_traj[(size_t)k * n + c] = (uint8_t)(jsel < 0 ? 255 : jsel);
+            }
+        }
         double pb = REF ? hyb(psn, hl_sfc) : fma(psn, hl_sfc.y, hl_sfc.x);
         if (pb < pref) { errbits |= PGW_ERR_PREF_BELOW_SFC; k_pref = min(k_pref, k); }
         if constexpr (REF) {
@@ -463,6 +563,7 @@ pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, co
     }
 
     // ---------------- phase 3: PS, QV of the parked levels, then the upper column ----------------
+    if constexpr (LOCAL) a.p_ref_out[c] = jsel < 0 ? (double)NAN : s_zgp[jsel];
     a.PS_out[c] = psn_f;
     a.dps_out[c] = (float)dps;
     {
@@ -529,6 +630,10 @@ pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, co
         if (a.first_k) {
             if (k_pref != INT32_MAX) atomicMin(a.first_k, k_pref);
             if (k_bound != INT32_MAX) atomicMin(a.first_k + 1, k_bound);
+            if constexpr (LOCAL) {
+                if (k_nopref != INT32_MAX) atomicMin(a.first_k + 2, k_nopref);
+                if (k_floor != INT32_MAX) atomicMin(a.first_k + 3, k_floor);
+            }
         }
     }
 }
@@ -539,7 +644,7 @@ __global__ void pgw_timestep_init_kernel(uint64_t *maxerr, float *stats, uint32_
     if (i == 0 && poly_fallback) *poly_fallback = 0u;
     if (i < PGW_MAX_ITER) maxerr[i] = 0ull;
     if (i < 2) stats[i] = INFINITY;
-    if (i < 2 && first_k) first_k[i] = INT32_MAX;
+    if (i < 4 && first_k) first_k[i] = INT32_MAX;
     if (i == 0) *err = 0u;
 }
 
@@ -557,8 +662,8 @@ __global__ void pgw_converge_kernel(const uint64_t *maxerr, int k_spec, double t
     res->reserved = 0;
 }
 
-// If the field converged before k_spec, PS and QV were written for dps_{k_spec};
-// rewrite them for dps_N.  e_pgw is recovered from the speculative QV.
+// If the field converged before k_spec, PS and QV (and p_ref) were written for iteration k_spec;
+// rewrite them for iteration N.  e_pgw is recovered from the speculative QV.
 __global__ void __launch_bounds__(256)
 pgw_rewrite_kernel(const __grid_constant__ pgw_timestep_args a, const pgw_timestep_result *res) {
     if (!res->rewritten) return;
@@ -566,6 +671,10 @@ pgw_rewrite_kernel(const __grid_constant__ pgw_timestep_args a, const pgw_timest
     const long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= n) return;
     const int N = res->n_iter;
+    if (a.flags & PGW_FLAG_LOCAL_PREF) {
+        const int j = a.pref_traj[(long long)(N - 1) * n + c];
+        a.p_ref_out[c] = j < a.nzg ? a.zg_plev[j] : (double)NAN;
+    }
     const double PSd = (double)a.PS[c];
     const double dps_n = (double)a.dps_traj[(long long)(N - 1) * n + c];
     const double dps_s = (double)a.dps_traj[(long long)(a.k_spec - 1) * n + c];
@@ -709,6 +818,12 @@ size_t column_smem(int nlev, int nplev, int np, int nt, bool ref) {
            (ref ? (size_t)np * nt * sizeof(float) : 0);                    // residual of the fp32 T_pgw
 }
 
+// PGW_FLAG_LOCAL_PREF: zg levels, candidates, the per-candidate ERA sums and the slot table (+ alignment)
+size_t local_pref_smem(int nzg, int ncand, int nt) {
+    return 16 + sizeof(double) * (size_t)(nzg + ncand) + 16 + 2 * sizeof(double) * (size_t)ncand * nt +
+           sizeof(int) * (size_t)nzg;
+}
+
 int validate(const pgw_timestep_args *a) {
     if (!a) return PGW_E_INVALID;
     if (a->ncol <= 0 || a->nlev < 2 || a->nplev < 2 || a->nplev > 64) return PGW_E_INVALID;
@@ -726,6 +841,13 @@ int validate(const pgw_timestep_args *a) {
     for (const void *p : need) if (!p) return PGW_E_INVALID;
     if ((reinterpret_cast<uintptr_t>(a->d4.lo) | reinterpret_cast<uintptr_t>(a->d4.hi)) & 15u) return PGW_E_INVALID;
     if (a->nsoil > 0 && (!a->T_SO || !a->T_SO_out)) return PGW_E_INVALID;
+    if (a->flags & PGW_FLAG_LOCAL_PREF) {
+        if (a->flags & PGW_FLAG_REF_DTYPES) return PGW_E_INVALID;
+        if (a->nzg < 1 || a->nzg > 64 || !(a->p_floor > 0.0)) return PGW_E_INVALID;
+        if ((unsigned long long)a->ncol * (unsigned long long)a->nzg >= (1ull << 31)) return PGW_E_INVALID;
+        if (!a->zg.lo || !a->zg.hi || !a->zg_plev || !a->zg_plev_host || !a->pref_traj || !a->p_ref_out)
+            return PGW_E_INVALID;
+    }
     return PGW_OK;
 }
 
@@ -737,14 +859,24 @@ bool tma_allowed() {
 
 pgw_column_plan plan_column(const pgw_timestep_args *a) {
     pgw_column_plan p;
-    p.lst = stash_top(a->ak_host, a->bk_host, a->nlev, a->p_ref, a->ps_bound);
+    p.local = (a->flags & PGW_FLAG_LOCAL_PREF) != 0;
+    // with a per-column p_ref the stash reaches up to the lowest p_ref it is sized for
+    const double p_stash = p.local ? a->p_floor : a->p_ref;
+    p.lst = stash_top(a->ak_host, a->bk_host, a->nlev, p_stash, a->ps_bound);
     p.np = a->nlev - p.lst;
     p.ref = (a->flags & PGW_FLAG_REF_DTYPES) != 0;
     p.smem = column_smem(a->nlev, a->nplev, p.np, kColumnThreads, p.ref);
+    p.ncand = 0;
+    if (p.local) {
+        for (int i = 0; i < a->nzg; ++i) p.ncand += a->zg_plev_host[i] >= a->p_floor;
+        p.smem += local_pref_smem(a->nzg, p.ncand, kColumnThreads);
+    }
     p.tma = false;
     int lst_tma = 0;
     size_t smem_tma = 0;
-    if (tma_allowed() && !(a->flags & (PGW_FLAG_DIRECT | PGW_FLAG_REF_DTYPES)) && pgw_tma_eligible(a, p.lst, &lst_tma, &smem_tma)) {
+    // the TMA flavour handles a scalar p_ref only
+    if (tma_allowed() && !(a->flags & (PGW_FLAG_DIRECT | PGW_FLAG_REF_DTYPES | PGW_FLAG_LOCAL_PREF)) &&
+        pgw_tma_eligible(a, p.lst, &lst_tma, &smem_tma)) {
         p.tma = true;
         p.lst = lst_tma;
         p.np = a->nlev - lst_tma;
@@ -754,7 +886,7 @@ pgw_column_plan plan_column(const pgw_timestep_args *a) {
     // [p_ref, ps_bound] (s is monotone in ps), so the series needs no exact-log fallback.
     p.fast = true;
     for (int l = p.lst; l < a->nlev; ++l)
-        for (double ps : {a->p_ref, a->ps_bound}) {
+        for (double ps : {p_stash, a->ps_bound}) {
             const double pt = a->ak_host[l] + ps * a->bk_host[l], pb = a->ak_host[l + 1] + ps * a->bk_host[l + 1];
             if (!(pt > 0.0) || !((pb - pt) / (pb + pt) < 0.055)) p.fast = false;
         }
@@ -785,13 +917,15 @@ int pgw_timestep(const pgw_timestep_args *a, void *stream) {
     pgw::pgw_timestep_init_kernel<<<1, 64, 0, st>>>(a->maxerr, a->stats, a->err, a->first_k, a->poly_fallback);
     if (plan.tma) return pgw_launch_column_tma(a, plan, st);
 
-    const int variant = plan.ref ? 2 : (plan.fast ? 1 : 0);
-    auto kern = plan.ref ? pgw::pgw_column_kernel<kColumnThreads, false, true>
-                         : (plan.fast ? pgw::pgw_column_kernel<kColumnThreads, true, false>
-                                      : pgw::pgw_column_kernel<kColumnThreads, false, false>);
+    const int variant = plan.local ? (plan.fast ? 9 : 8) : plan.ref ? 2 : (plan.fast ? 1 : 0);
+    auto kern = plan.local ? (plan.fast ? pgw::pgw_column_kernel<kColumnThreads, true, false, true>
+                                        : pgw::pgw_column_kernel<kColumnThreads, false, false, true>)
+              : plan.ref   ? pgw::pgw_column_kernel<kColumnThreads, false, true>
+                           : (plan.fast ? pgw::pgw_column_kernel<kColumnThreads, true, false>
+                                        : pgw::pgw_column_kernel<kColumnThreads, false, false>);
     if ((rc = pgw_ensure_smem((const void *)kern, variant, plan.smem, plan.np)) != PGW_OK) return rc;
     const unsigned grid = (unsigned)((a->ncol + kColumnThreads - 1) / kColumnThreads);
-    kern<<<grid, kColumnThreads, plan.smem, st>>>(*a, plan.lst, plan.np);
+    kern<<<grid, kColumnThreads, plan.smem, st>>>(*a, plan.lst, plan.np, plan.ncand);
     return pgw_check_launch("pgw_column_kernel");
 }
 

@@ -212,11 +212,14 @@ class PGWEngine:
     """
     ak, bk: half-level hybrid coefficients [L+1] (index 0 = model top); akm/bkm
     optional full-level coefficients (else the reference's mid-point rule,
-    step_03_apply_to_era.py:68-85); soil1: soil depths [S].
+    step_03_apply_to_era.py:68-85); soil1: soil depths [S].  ``ps_bound`` and, with
+    ``p_ref_inp = None``, ``p_floor`` (the lowest per-column reference pressure) size the
+    column stash; a timestep that leaves that range is rerun with a wider one.  The default
+    floor of 300 hPa is a lower pressure than the ~400 hPa the highest ERA5 terrain selects.
     """
 
     def __init__(self, ak, bk, deltas, soil1=(), akm=None, bkm=None, ps_bound=110000.0, group=None,
-                 band_exchange="auto"):
+                 band_exchange="auto", p_floor=30000.0):
         if not torch.cuda.is_available():
             raise RuntimeError("PGWEngine needs a CUDA device (B200, sm_100a); there is no CPU path")
         self.deltas = deltas
@@ -238,6 +241,8 @@ class PGWEngine:
             raise ValueError("at most %d soil levels" % N.PGW_MAX_SOIL)
         self.soil_decay = np.exp(-soil1 / 2.8).astype(np.float64)     # step_03:140
         self.ps_bound = float(ps_bound)
+        self.p_floor = float(p_floor)
+        self._zg_tables = None
         self.group = group
         # latitude-band mode: how the bands agree on the iteration count.  "p2p": pgw_band_exchange, one kernel over
         # peer memory behind the column kernel (inboxes in torch symmetric memory); "nccl": pack, all-reduce(MAX),
@@ -319,8 +324,9 @@ class PGWEngine:
         T, QV, U, V [1,L,ny,nx] (the names of settings.var_name_map).  Returns a
         ``Pending``; nothing is synchronised here.
         """
-        if settings.i_reinterp or settings.p_ref_inp is None:
-            raise ValueError("i_reinterp = 1 / p_ref_inp = None run through the staged path: use apply()")
+        if settings.i_reinterp or (settings.p_ref_inp is None and getattr(settings, "i_reference_dtypes", 0)):
+            raise ValueError("i_reinterp = 1 / p_ref_inp = None with i_reference_dtypes = 1 run through the "
+                             "staged path: use apply()")
         a, f, out, ws, k_spec, k_max = self._fill_args(era, era_step_dt, out, k_spec, slot)
         if direct:
             a.flags |= N.FLAG_DIRECT          # every parked level integrated in every iteration
@@ -359,7 +365,7 @@ class PGWEngine:
         ws["event"].record()
         ctx = dict(era=era, when=era_step_dt, ignore_top=ignore_top_pressure_error, k_spec=k_spec,
                    k_max=k_max, keep=(f, a), file_name=file_name, slot=slot, direct=direct,
-                   stream=torch.cuda.current_stream())
+                   stream=torch.cuda.current_stream(), local_pref=bool(a.flags & N.FLAG_LOCAL_PREF))
         p = Pending(self, a, out, ws, ctx)
         ws["inflight"] = p
         return p
@@ -396,8 +402,11 @@ class PGWEngine:
         ws = self._workspace(ncol, k_max, slot)
 
         zg = ds.vars["zg"]
-        if settings.p_ref_inp is None:                                    # staged path: level picked per column
+        local = settings.p_ref_inp is None                                # level picked per column and iteration
+        if local:
             sel0, p_ref_scalar = 0, float(zg["plev"][0])
+            if "p_ref" not in out:
+                out["p_ref"] = torch.empty((1, ny, nx), device=self.device, dtype=torch.float64)
         else:
             p_ref_scalar = float(settings.p_ref_inp)
             sel0 = self._zg_level.get(p_ref_scalar)
@@ -454,6 +463,21 @@ class PGWEngine:
         a.k_spec = k_spec
         a.ps_bound = self.ps_bound
         a.flags = N.FLAG_REF_DTYPES if getattr(settings, "i_reference_dtypes", 0) else 0
+        if local:
+            if self._zg_tables is None:
+                plev = np.ascontiguousarray(zg["plev"], dtype=np.float64)
+                if len(np.unique(plev)) != len(plev):
+                    raise ValueError("zg pressure levels must be distinct")
+                self._zg_tables = (plev, torch.as_tensor(plev, device=self.device))
+            plev, plev_d = self._zg_tables
+            a.flags |= N.FLAG_LOCAL_PREF
+            a.zg = ds.slab("zg", era_step_dt)
+            a.zg_plev, a.zg_plev_host, a.nzg = plev_d.data_ptr(), plev.ctypes.data, len(plev)
+            a.p_floor = self.p_floor
+            if "pref_traj" not in ws:
+                ws["pref_traj"] = torch.empty(ws["traj"].shape, device=self.device, dtype=torch.uint8)
+            a.pref_traj = ws["pref_traj"].data_ptr()
+            a.p_ref_out = out["p_ref"].data_ptr()
         return a, f, out, ws, k_spec, k_max
 
     # ------------------------------------------------------------------ completion
@@ -471,6 +495,15 @@ class PGWEngine:
             err &= ~N.ERR_PREF_BELOW_SFC
         if (err & N.ERR_PS_BOUND) and st.first_k[1] >= n_ran:
             err &= ~N.ERR_PS_BOUND
+        if (err & N.ERR_NO_PREF) and st.first_k[2] >= n_ran:
+            err &= ~N.ERR_NO_PREF
+        if (err & N.ERR_PREF_FLOOR) and st.first_k[3] >= n_ran:
+            err &= ~N.ERR_PREF_FLOOR
+        # a column that left the stash computes garbage from then on, which can end in NO_PREF later: rerun first
+        k_stash = min(st.first_k[1] if err & N.ERR_PS_BOUND else N.INT32_MAX,
+                      st.first_k[3] if err & N.ERR_PREF_FLOOR else N.INT32_MAX)
+        if (err & N.ERR_NO_PREF) and st.first_k[2] > k_stash:
+            err &= ~N.ERR_NO_PREF
         if err & N.ERR_BAND_TIMEOUT:
             raise RuntimeError("latitude-band exchange: the status block of a peer rank did not arrive")
         if err & N.ERR_PS_HIST_RANGE:
@@ -478,10 +511,17 @@ class PGWEngine:
         if (min_targ_p < min_src_p or min_targ_p < float(np.min(self.deltas.plev))) \
                 and not ctx["ignore_top"]:
             raise ValueError(MSG_TOP)                                    # functions.py:417-425
+        if err & N.ERR_NO_PREF:
+            from .staged import MSG_NO_PREF
+            raise ValueError(MSG_NO_PREF)                                # step_03:245-251
         if err & N.ERR_PREF_BELOW_SFC:
             raise ValueError(MSG_PREF)                                   # functions.py:162-165
-        if err & N.ERR_PS_BOUND:
-            self.ps_bound *= 1.25
+        if err & (N.ERR_PS_BOUND | N.ERR_PREF_FLOOR):
+            if err & N.ERR_PS_BOUND:
+                self.ps_bound *= 1.25
+            if err & N.ERR_PREF_FLOOR:                                   # one more zg level into the stash
+                below = self._zg_tables[0][self._zg_tables[0] < self.p_floor]
+                self.p_floor = float(below.max()) if len(below) else 0.8 * self.p_floor
             self.stats["reruns"] += 1
             with torch.cuda.stream(ctx["stream"]):       # a rerun goes where the timestep was submitted
                 return self.submit(ctx["era"], ctx["when"], out=p.out, ignore_top_pressure_error=ctx["ignore_top"],
@@ -505,14 +545,17 @@ class PGWEngine:
         res["n_iter"] = int(n_iter)
         res["phi_max_errors"] = [float(x) for x in maxerr[:int(n_iter)]]
         res["poly_fallback"] = int(st.poly_fallback)
+        if not ctx.get("local_pref"):
+            res.pop("p_ref", None)
         if settings.i_debug >= 2:
             for it, e in enumerate(res["phi_max_errors"], 1):
                 print("### iteration {:03d}, phi max error: {}".format(it, e))
         return res
 
     def apply(self, era, era_step_dt, **kw):
-        """Synchronous form of ``submit``: returns the output dict (device tensors).  The settings
-        the fused pass does not cover (i_reinterp = 1, p_ref_inp = None) take the staged path."""
+        """Synchronous form of ``submit``: returns the output dict (device tensors).  i_reinterp = 1,
+        which the fused pass does not cover, and p_ref_inp = None take the staged path (``submit``
+        runs p_ref_inp = None in the fused pass)."""
         if settings.i_reinterp or settings.p_ref_inp is None:
             from . import staged
             kw.pop("k_spec", None)

@@ -59,7 +59,7 @@ nan_interp_kernel_radius = 1000000  # m
 nan_interp_sharpness = 4
 
 # surface-pressure adjustment
-p_ref_inp = 30000  # Pa; None = choose locally (not on the CUDA path yet)
+p_ref_inp = 30000  # Pa; None = choose locally (PGWEngine.submit: fused kernel; apply: staged path)
 adj_factor = 0.95
 thresh_phi_ref_max_error = 0.15
 max_n_iter = 20
