@@ -27,9 +27,10 @@
 extern "C" {
 #endif
 
-#define PGW_B200_ABI_VERSION 7   /* 6: + pgw_timestep_status, pgw_timestep_run/_finish, PGW_FLAG_REF_DTYPES, first_k,
+#define PGW_B200_ABI_VERSION 8   /* 6: + pgw_timestep_status, pgw_timestep_run/_finish, PGW_FLAG_REF_DTYPES, first_k,
                                        pgw_band_pack/_unpack, pgw_band_exchange, pgw_regrid_bilinear_band_f32
-                                    7: + PGW_FLAG_LOCAL_PREF and its args, PGW_ERR_PREF_FLOOR, first_k[4] */
+                                    7: + PGW_FLAG_LOCAL_PREF and its args, PGW_ERR_PREF_FLOOR, first_k[4]
+                                    8: + PGW_FLAG_REINTERP (no layout change) */
 
 /* host-side return codes */
 #define PGW_OK               0
@@ -74,6 +75,19 @@ extern "C" {
                                 cp.async flavour; not combinable with PGW_FLAG_REF_DTYPES.  Reads the last block of
                                 pgw_timestep_args (zg .. p_ref_out); p_ref and zg_ref are ignored, p_floor sizes the
                                 column stash in place of p_ref. */
+#define PGW_FLAG_REINTERP 8   /* i_reinterp = 1 (step_03_apply_to_era.py:155-173, :202-216, :330-343): no delta is
+                                applied before the iteration; every iteration interpolates the ERA state (T, RELHUM)
+                                linearly in ln p ('constant' extrapolation, functions.py:434-580) onto its own
+                                pressures akm + ps_pgw bkm and adds the deltas there, and ta_pgw of the lowest level
+                                of that iteration divides adj_ps.  The outputs are the state evaluated in the last
+                                iteration: PS, and T, QV, U, V on every level at its pressures (U, V interpolated
+                                after the loop).  Takes the cp.async flavour; not combinable with
+                                PGW_FLAG_LOCAL_PREF or PGW_FLAG_REF_DTYPES (PGW_E_INVALID).  When N < k_spec,
+                                pgw_timestep_finalize does not rewrite PS/QV from the speculative QV: it relaunches
+                                the column kernel with k_spec = N read from the device result (a replay: every CTA
+                                returns at once unless `rewritten` is set; its updates of maxerr, err, first_k and
+                                stats repeat values already there), so the outputs equal those of a run with
+                                k_spec = N bit for bit. */
 
 #define PGW_MAX_SOIL   16
 #define PGW_MAX_ITER   64
@@ -194,7 +208,8 @@ int pgw_time_mean_f32(const float *series, int ntime, float *out, long long n, v
 /* ------------------------------------------------------------------------
  * The fused per-timestep pass.
  * Replaces the body of pgw_for_era5(), step_03_apply_to_era.py:60-343 with
- * i_reinterp = 0 and a scalar or (PGW_FLAG_LOCAL_PREF) per-column p_ref: pressures (:64-88), RELHUM (:91-94),
+ * a scalar or (PGW_FLAG_LOCAL_PREF, i_reinterp = 0) per-column p_ref, and i_reinterp = 0 or
+ * (PGW_FLAG_REINTERP) 1: pressures (:64-88), RELHUM (:91-94),
  * sea-ice/skin/soil update (:103-146, integrate_tos), load_delta's time blend
  * (functions.py:288-292), replace_delta_sfc + vert_interp_delta
  * (functions.py:343-431) for ta,hur,ua,va, delta application (:158-173) and
@@ -208,7 +223,8 @@ int pgw_time_mean_f32(const float *series, int ntime, float *out, long long n, v
  * dps_k in dps_traj, and writes PS/QV for dps_{k_spec}.  The caller then
  *   - all-reduces maxerr (MAX) over ranks in latitude-band mode,
  *   - calls pgw_timestep_finalize(), which finds N on the device and, if
- *     N < k_spec, rewrites PS/QV for dps_N,
+ *     N < k_spec, rewrites PS/QV for dps_N (PGW_FLAG_REINTERP: replays the
+ *     column kernel for k_spec = N),
  *   - reruns with a larger k_spec if maxerr[k_spec-1] > thresh.
  * ---------------------------------------------------------------------- */
 typedef struct pgw_tslab {
@@ -294,7 +310,8 @@ long long pgw_sizeof_timestep_args(void);   /* for FFI layout checks */
 long long pgw_timestep_smem_bytes(const pgw_timestep_args *a);
 /* 1 if pgw_timestep() takes the TMA flavour of the column kernel for these args, 0 if the
  * per-thread cp.async flavour (odd ncol, unaligned fields, PGW_COLUMN_PATH=generic, PGW_FLAG_DIRECT,
- * PGW_FLAG_REF_DTYPES, and PGW_FLAG_LOCAL_PREF on every grid: the TMA flavour handles a scalar p_ref only) */
+ * PGW_FLAG_REF_DTYPES, and PGW_FLAG_LOCAL_PREF and PGW_FLAG_REINTERP on every grid: the TMA flavour handles a
+ * scalar p_ref and iteration-invariant parked levels only) */
 int pgw_timestep_uses_tma(const pgw_timestep_args *a);
 int pgw_timestep(const pgw_timestep_args *a, void *stream);
 
@@ -353,8 +370,9 @@ int pgw_band_exchange(pgw_timestep_status *status_dev, double *const *inbox_ptrs
 /* ------------------------------------------------------------------------
  * The staged per-timestep path: pgw_for_era5() run stage by stage on float64
  * device arrays with the operators above plus the small ones below.  It covers
- * i_reinterp = 1 (step_03_apply_to_era.py:202-216, :330-343), which the fused pass does not, and
- * p_ref_inp = None (:219-251), the reference the fused pass's PGW_FLAG_LOCAL_PREF is tested against;
+ * i_reinterp = 1 (step_03_apply_to_era.py:202-216, :330-343) and p_ref_inp = None (:219-251), the references
+ * the fused pass's PGW_FLAG_REINTERP and PGW_FLAG_LOCAL_PREF are tested against, and their combination with
+ * each other or with the file dtypes, which the fused pass does not cover;
  * host orchestration: pgw4era5_b200/staged.py.
  *   pgw_surface_update        sea ice / skin / soil block, step_03:103-146
  *                             (reads only the 2-D members of the args)

@@ -32,6 +32,7 @@ BAND_PARITIES = 8
 FLAG_DIRECT = 1
 FLAG_REF_DTYPES = 2
 FLAG_LOCAL_PREF = 4
+FLAG_REINTERP = 8
 RUN_NO_FINALIZE = 1
 BAND_WORDS = 64 + 2 + 32 + 4
 INT32_MAX = 2 ** 31 - 1
@@ -72,7 +73,7 @@ class TimestepStatus(C.Structure):
                 ("err", C.c_uint32), ("first_k", C.c_int32 * 4), ("poly_fallback", C.c_uint32)]
 
 
-ABI_VERSION = 7          # PGW_B200_ABI_VERSION of include/pgw_b200.h
+ABI_VERSION = 8          # PGW_B200_ABI_VERSION of include/pgw_b200.h
 
 
 class NativeError(RuntimeError):

@@ -193,6 +193,23 @@ __device__ __forceinline__ float2 thermo_e_pgw_x2(bool cold, float2 p, float2 t,
 }
 __device__ __forceinline__ bool is_cold(float t, float dta) { return fmaxf(t, t + dta) <= 250.0f; }   // conservative
 
+// Saturation vapour pressure over water and ice (functions.py:74-105) of ONE state, given as T - 273: the
+// general (not `cold`) form of thermo_e_pgw.  PGW_FLAG_REINTERP, whose levels are not swept in warp-uniform pairs.
+__device__ __forceinline__ float es_water_ice(float tm273) {
+    const float dT = tm273 - 0.16f;
+    constexpr float kCw = 17.502f * 1.4426950408889634f, kCi = 22.587f * 1.4426950408889634f;
+    const float dw = tm273 + (273.0f - 32.19f), di = tm273 + (273.0f + 0.7f);
+    const float rr = fast_rcp(dw * di);
+    const float ew = fast_ex2(kCw * dT * (rr * di)), ei = fast_ex2(kCi * dT * (rr * dw));
+    const float r = (dT + 23.0f) * (1.0f / 23.0f);
+    const float al = dT >= 0.0f ? 1.0f : (dT <= -23.0f ? 0.0f : r * r);              // NaN stays NaN
+    return 611.21f * (al * ew + (1.0f - al) * ei);
+}
+// RELHUM of the ERA state (step_03_apply_to_era.py:91-94, functions.py:107-116) at p = akm + PS * bkm
+__device__ __forceinline__ float rh_era_f32(float p, float t, float q) {
+    return 100.0f * q * p * fast_rcp((0.622f + 0.378f * q) * es_water_ice(t - 273.0f));
+}
+
 // specific humidity from vapour pressure (functions.py:66-72), p = akm + ps * bkm
 __device__ __forceinline__ float qv_from_e(float e, float ps, float2 m) {
     return 0.622f * e * fast_rcp(fmaf(-0.378f, e, fmaf(ps, m.y, m.x)));
@@ -295,6 +312,7 @@ struct pgw_column_plan {
     bool fast;          // ln_ratio series valid for every layer the iteration can touch
     bool local;         // PGW_FLAG_LOCAL_PREF
     int ncand;          // PGW_FLAG_LOCAL_PREF: zg levels >= p_floor (candidate p_ref levels)
+    bool reinterp;      // PGW_FLAG_REINTERP
 };
 // pgw_column_tma.cu
 bool pgw_tma_eligible(const pgw_timestep_args *a, int lst_generic, int *lst_tma, size_t *smem);

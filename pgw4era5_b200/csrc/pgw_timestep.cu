@@ -47,10 +47,23 @@ constexpr int kRing = 5;     // levels in flight per thread (cp.async ring, +1 s
 // LOCAL: PGW_FLAG_LOCAL_PREF, p_ref per column and iteration among zg's levels (step_03:219-251).  Phase 1
 // records the ERA-state sums at every candidate level (the `ncand` zg levels >= p_floor) the column's p_ref can
 // move up to; phase 2 re-picks p_ref in every iteration and integrates the parked levels up to it.
-template <int NT, bool FAST, bool REF, bool LOCAL = false>
+// RI: PGW_FLAG_REINTERP, i_reinterp = 1 (step_03:155-173, :202-216, :330-343).  The stash holds the ERA state
+// (T, RELHUM); every iteration after the first re-interpolates it, in ln p, onto that iteration's pressures
+// and adds the deltas there.  `replay` (RI only, else null): pgw_timestep_finalize's relaunch that rewrites the
+// outputs for iteration N when the speculative run went further (see PGW_FLAG_REINTERP in the header).
+template <int NT, bool FAST, bool REF, bool LOCAL = false, bool RI = false>
 __global__ void __launch_bounds__(NT, REF ? 2 : 3)
-pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, const int np, const int ncand) {
+pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, const int np, const int ncand,
+                  const pgw_timestep_result *replay) {
     static_assert(!(REF && LOCAL), "PGW_FLAG_LOCAL_PREF runs with float64 accumulation only");
+    static_assert(!(RI && (REF || LOCAL)), "PGW_FLAG_REINTERP runs with a scalar p_ref and float64 accumulation");
+    int k_spec = a.k_spec;
+    if constexpr (RI) {
+        if (replay) {                       // the same word for every thread: the whole grid returns or runs
+            if (!replay->rewritten) return;
+            k_spec = replay->n_iter;
+        }
+    }
     extern __shared__ __align__(16) unsigned char smem[];
     const int L = a.nlev, K = a.nplev;
     // ---- shared memory carve-up
@@ -184,7 +197,8 @@ pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, co
     };
 
     Walk2 wA, wB;
-    {
+    // Both walkers at the bottom of the column (RI: again at the start of every iteration's sweep).
+    auto init_walkers = [&]() {
         // replace_delta_sfc: node s carries (ps_hist, surface delta); the nodes after it all
         // hold the surface delta, so node s acts as the last node of the column.
         const float psh = (float)blend_f64(a.ps_hist, r_psh);
@@ -216,7 +230,8 @@ pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, co
             if (s - d >= 0) l2_prefetch(0, s - d);
             if (K - 1 - d >= 0) l2_prefetch(1, K - 1 - d);
         }
-    }
+    };
+    init_walkers();
     float min_src_p = (wA.lo == 0) ? wA.p_lo : s_plev[0];
 
     // One downward step of a walker, split in two so that the steps of both walkers can be
@@ -317,6 +332,9 @@ pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, co
     // geopotential as Rd * sum_l r_l dlnp_l; that sum is taken once with the ERA pressures
     // (its change over the iteration is < 1e-8 m2/s2) and added to every iteration's sum.
     double acc_res = 0.0, acc_pgw0 = 0.0, t_low_d = 0.0;
+    // RI: the state of iteration 1 is the output only when it is the last one; later ones are written by the
+    // last iteration's sweep
+    const bool out1 = !RI || k_spec == 1;
     {
         float2 *pTe = st_Te + (size_t)(L - 1 - lst) * NT + tid;
         // ERA geopotential of one layer (functions.py:128-189), sequential in the column
@@ -394,10 +412,18 @@ pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, co
             const bool cold = __all_sync(0xffffffffu, is_cold(t0, d0.ta) && is_cold(t1, d1.ta));
             const float e0 = thermo(cold, p0, t0, q0, d0), e1 = thermo(cold, p1, t1, q1, d1);
             const float tp0 = t0 + d0.ta, tp1 = t1 + d1.ta;   // == (float)((double)t + (double)dta)
-            st_stream(oT + off, tp0); st_stream(oU + off, u0 + d0.ua); st_stream(oV + off, v0 + d0.va);
-            st_stream(oT + off - n, tp1); st_stream(oU + off - n, u1 + d1.ua); st_stream(oV + off - n, v1 + d1.va);
-            pTe[0] = make_float2(tp0, e0);
-            pTe[-NT] = make_float2(tp1, e1);
+            if (out1) {
+                st_stream(oT + off, tp0); st_stream(oU + off, u0 + d0.ua); st_stream(oV + off, v0 + d0.va);
+                st_stream(oT + off - n, tp1); st_stream(oU + off - n, u1 + d1.ua); st_stream(oV + off - n, v1 + d1.va);
+                if constexpr (RI) { st_stream(oQ + off, qv_from_e(e0, ps_f, m0)); st_stream(oQ + off - n, qv_from_e(e1, ps_f, m1)); }
+            }
+            if constexpr (RI) {
+                pTe[0] = make_float2(t0, rh_era_f32(p0, t0, q0));
+                pTe[-NT] = make_float2(t1, rh_era_f32(p1, t1, q1));
+            } else {
+                pTe[0] = make_float2(tp0, e0);
+                pTe[-NT] = make_float2(tp1, e1);
+            }
             if (l == L - 1) t_low_d = (double)t0 + (double)d0.ta;
             era_layer(l, p0, t0, q0, d0.ta, tp0, e0);
             era_layer(l - 1, p1, t1, q1, d1.ta, tp1, e1);
@@ -413,8 +439,12 @@ pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, co
             const Dlt d0 = walk(p0);
             const float e0 = thermo(false, p0, t0, q0, d0);
             const float tp0 = t0 + d0.ta;
-            st_stream(oT + off, tp0); st_stream(oU + off, u0 + d0.ua); st_stream(oV + off, v0 + d0.va);
-            pTe[0] = make_float2(tp0, e0);
+            if (out1) {
+                st_stream(oT + off, tp0); st_stream(oU + off, u0 + d0.ua); st_stream(oV + off, v0 + d0.va);
+                if constexpr (RI) st_stream(oQ + off, qv_from_e(e0, ps_f, m0));
+            }
+            if constexpr (RI) pTe[0] = make_float2(t0, rh_era_f32(p0, t0, q0));
+            else pTe[0] = make_float2(tp0, e0);
             if (l == L - 1) t_low_d = (double)t0 + (double)d0.ta;
             era_layer(l, p0, t0, q0, d0.ta, tp0, e0);
             off -= n;
@@ -441,14 +471,84 @@ pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, co
         else phi_era = NAN;
     }
     const float2 *const bTe = st_Te + (size_t)(L - 1 - lst) * NT + tid;  // lowest level of the stash
-    const double t_low = t_low_d;                                 // ta_pgw on the lowest level
+    double t_low = t_low_d;                                       // ta_pgw on the lowest level (RI: per iteration)
 
     // ---------------- phase 2: surface-pressure fixed point (step_03:182-319) ----------------
     // The loads of the upper column are already in flight and overlap this phase.
     double dps = 0.0, adj = 0.0, psn = PSd;
     int ltop = lst + 1;                 // first layer (from the top) lying entirely below p_ref
+
+    // RI: the ERA state at a target pressure of this iteration, interp_logp_4d in 'constant' mode
+    // (functions.py:434-580, float64): a merge walk over the ERA levels (pressures akm + PS bkm) as the targets
+    // move up the column.  lo = level rj, hi = level rj + 1.  A level comes from the stash, or from global
+    // memory above it (a target lowered by dps < 0 brackets with level lst - 1) or in phase 3; U and V, needed
+    // for the outputs only, from global memory.  Level `lring` takes (t, q, u, v) just read from the ring.
+    struct Era { double pe; float t, r, u, v; };
+    int rj = L - 1;
+    Era elo{}, ehi{};
+    double inv_den = 0.0;                                         // 1 / ln(p_hi / p_lo)
+    auto era_at = [&](int j, bool uv, int lring, float t, float q, float u, float v) {
+        Era x;
+        x.pe = fma(PSd, __ldg(a.bkm + j), __ldg(a.akm + j));
+        const uint32_t o = (uint32_t)j * n + c;
+        if (j >= lst) {
+            const float2 s = st_Te[(size_t)(j - lst) * NT + tid];
+            x.t = s.x; x.r = s.y;
+        } else {
+            const float2 m = s_m[j];
+            if (j != lring) { t = __ldg(gT + o); q = __ldg(gQ + o); }
+            x.t = t;
+            x.r = rh_era_f32(fmaf(ps_f, m.y, m.x), t, q);
+        }
+        if (uv && j != lring) { u = __ldg(gU + o); v = __ldg(gV + o); }
+        x.u = uv ? u : 0.0f;
+        x.v = uv ? v : 0.0f;
+        return x;
+    };
+    auto win_reset = [&](int j, bool uv) { rj = j; elo = era_at(j, uv, -1, 0.0f, 0.0f, 0.0f, 0.0f); };
+    // move the window down to target pt; returns the weight of hi, 0 for lo's value as it is (an exact hit,
+    // or constant extrapolation below level L-1 or above level 0)
+    auto win_move = [&](double pt, bool uv, int lring, float t, float q, float u, float v) -> double {
+        while (rj > 0 && elo.pe > pt) {
+            ehi = elo;
+            --rj;
+            elo = era_at(rj, uv, lring, t, q, u, v);
+            inv_den = 1.0 / ln_ratio<false>(ehi.pe, elo.pe, lk);
+        }
+        // ln(pt / p_lo) from pt - p_lo (= bkm dps on the level itself): no float32 log of a ratio near 1
+        return (rj == L - 1 || !(elo.pe < pt)) ? 0.0 : ln_ratio<false>(pt, elo.pe, lk) * inv_den;
+    };
+    auto lerp = [](double w, float lo, float hi) {
+        return w == 0.0 ? (double)lo : fma(w, (double)hi - (double)lo, (double)lo);
+    };
+    // level l at this iteration's pressures: T_pgw (float64), e and 1/(p - 0.378 e) (functions.py:118-125),
+    // with `uv` also U and V
+    struct RiLev { double tp, u, v; float e, g; };
+    auto ri_level = [&](int l, bool uv, int lring, float t, float q, float u, float v) {
+        const double pt = fma(psn, __ldg(a.bkm + l), __ldg(a.akm + l));
+        const float2 m = s_m[l];
+        const float ptf = fmaf(psn_f, m.y, m.x);
+        const double w = win_move(pt, uv, lring, t, q, u, v);
+        const Dlt d = walk(ptf);
+        RiLev r;
+        r.tp = lerp(w, elo.t, ehi.t) + (double)d.ta;
+        const float rh = (float)(lerp(w, elo.r, ehi.r) + (double)d.hur);
+        r.e = rh * 0.01f * es_water_ice((float)(r.tp - 273.0));
+        r.g = fast_rcp(fmaf(-0.378f, r.e, ptf));
+        r.u = uv ? lerp(w, elo.u, ehi.u) + (double)d.ua : 0.0;
+        r.v = uv ? lerp(w, elo.v, ehi.v) + (double)d.va : 0.0;
+        return r;
+    };
+    auto ri_store = [&](int l, const RiLev &r) {
+        const uint32_t o = (uint32_t)l * n + c;
+        st_stream(oT + o, (float)r.tp);
+        st_stream(oQ + o, 0.622f * r.e * r.g);
+        st_stream(oU + o, (float)r.u);
+        st_stream(oV + o, (float)r.v);
+    };
+
     float *traj = a.dps_traj + c;
-    for (int k = 0; k < a.k_spec; ++k, traj += n) {
+    for (int k = 0; k < k_spec; ++k, traj += n) {
         if constexpr (REF) {
             // delta_ps is float32 (zeros_like(PS)) and += keeps that; ps_pgw = PS + delta_ps is a float32 sum
             // (step_03_apply_to_era.py:186-195)
@@ -522,6 +622,32 @@ pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, co
         double acc = acc_res;
         if (k == 0) {
             acc += acc_pgw0;            // psn == PS: summed in phase 1 together with the ERA state
+        } else if constexpr (RI) {
+            // re-interpolate the parked levels bottom-up to the layer that contains p_ref (step_03:202-216);
+            // the last iteration goes on over every parked level and writes its state
+            const bool last = k == k_spec - 1;
+            init_walkers();
+            win_reset(L - 1, last);
+            acc = 0.0;                  // T_pgw is formed in float64: no fp32 residual
+            bool open = pb >= pref;
+            for (int l = L - 1; l >= lst; --l) {
+                const RiLev r = ri_level(l, last, -1, 0.0f, 0.0f, 0.0f, 0.0f);
+                if (l == L - 1) t_low = r.tp;                           // ta_pgw[:, -1] of this iteration
+                if (open) {
+                    const double tv = fma(r.tp, (double)((0.61f * 0.622f) * r.e * r.g), r.tp);
+                    const double2 hl = s_hl[l];
+                    const double pt = fma(psn, hl.y, hl.x);
+                    if (pt < pref) {                                    // layer that contains p_ref (:174-179)
+                        acc = fma(tv, ln_ratio<FAST>(pb, pref, lk), acc);
+                        open = false;
+                    } else {
+                        acc = fma(tv, ln_ratio<FAST>(pb, pt, lk), acc);
+                        pb = pt;
+                    }
+                }
+                if (last) ri_store(l, r);
+                else if (!open) break;
+            }
         } else {
         // layers ltop..L-1 are entirely below p_ref for this ps; it moves by at most a level or two
         while (ltop > lst) { const double2 h = s_hl[ltop - 1]; if (fma(psn, h.y, h.x) >= pref) --ltop; else break; }
@@ -566,6 +692,19 @@ pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, co
     if constexpr (LOCAL) a.p_ref_out[c] = jsel < 0 ? (double)NAN : s_zgp[jsel];
     a.PS_out[c] = psn_f;
     a.dps_out[c] = (float)dps;
+    if constexpr (RI) {
+        // the upper column at the final pressures (step_03:330-343 for U and V); the window goes on from the
+        // top of the stash (the last sweep left it there; with one iteration, place it there)
+        if (k_spec == 1) win_reset(lst, true);
+        for (int l = lst - 1; l >= 0; --l) {
+            __pipeline_wait_prior(kRing - 1);
+            const float *sl0 = my_ring + slot_r * (4 * NT);
+            const float t0 = sl0[0], q0 = sl0[NT], u0 = sl0[2 * NT], v0 = sl0[3 * NT];
+            slot_r = (slot_r == kRing) ? 0 : slot_r + 1;
+            prefetch();                                  // overwrites the slot read one level ago
+            ri_store(l, ri_level(l, true, l, t0, q0, u0, v0));
+        }
+    } else {
     {
         const float2 *pTe = bTe;
         uint32_t o2 = (uint32_t)(L - 1) * n + c;
@@ -615,10 +754,12 @@ pgw_column_kernel(const __grid_constant__ pgw_timestep_args a, const int lst, co
             off -= n;
         }
     }
+    }
     __pipeline_wait_prior(0);
 
     // ---------------- bookkeeping for the host-side checks ----------------
     float p_top = fmaf(ps_f, s_m[0].y, s_m[0].x);                        // functions.py:417
+    if constexpr (RI) p_top = fminf(p_top, fmaf(psn_f, s_m[0].y, s_m[0].x));    // targets of the last iteration
     p_top = warp_min(p_top);
     min_src_p = warp_min(min_src_p);
     if ((tid & 31) == 0) {
@@ -841,6 +982,7 @@ int validate(const pgw_timestep_args *a) {
     for (const void *p : need) if (!p) return PGW_E_INVALID;
     if ((reinterpret_cast<uintptr_t>(a->d4.lo) | reinterpret_cast<uintptr_t>(a->d4.hi)) & 15u) return PGW_E_INVALID;
     if (a->nsoil > 0 && (!a->T_SO || !a->T_SO_out)) return PGW_E_INVALID;
+    if ((a->flags & PGW_FLAG_REINTERP) && (a->flags & (PGW_FLAG_LOCAL_PREF | PGW_FLAG_REF_DTYPES))) return PGW_E_INVALID;
     if (a->flags & PGW_FLAG_LOCAL_PREF) {
         if (a->flags & PGW_FLAG_REF_DTYPES) return PGW_E_INVALID;
         if (a->nzg < 1 || a->nzg > 64 || !(a->p_floor > 0.0)) return PGW_E_INVALID;
@@ -865,6 +1007,7 @@ pgw_column_plan plan_column(const pgw_timestep_args *a) {
     p.lst = stash_top(a->ak_host, a->bk_host, a->nlev, p_stash, a->ps_bound);
     p.np = a->nlev - p.lst;
     p.ref = (a->flags & PGW_FLAG_REF_DTYPES) != 0;
+    p.reinterp = (a->flags & PGW_FLAG_REINTERP) != 0;
     p.smem = column_smem(a->nlev, a->nplev, p.np, kColumnThreads, p.ref);
     p.ncand = 0;
     if (p.local) {
@@ -874,8 +1017,9 @@ pgw_column_plan plan_column(const pgw_timestep_args *a) {
     p.tma = false;
     int lst_tma = 0;
     size_t smem_tma = 0;
-    // the TMA flavour handles a scalar p_ref only
-    if (tma_allowed() && !(a->flags & (PGW_FLAG_DIRECT | PGW_FLAG_REF_DTYPES | PGW_FLAG_LOCAL_PREF)) &&
+    // the TMA flavour handles a scalar p_ref only, and parks (T_pgw, e_pgw) that do not change over the iteration
+    if (tma_allowed() &&
+        !(a->flags & (PGW_FLAG_DIRECT | PGW_FLAG_REF_DTYPES | PGW_FLAG_LOCAL_PREF | PGW_FLAG_REINTERP)) &&
         pgw_tma_eligible(a, p.lst, &lst_tma, &smem_tma)) {
         p.tma = true;
         p.lst = lst_tma;
@@ -891,6 +1035,18 @@ pgw_column_plan plan_column(const pgw_timestep_args *a) {
             if (!(pt > 0.0) || !((pb - pt) / (pb + pt) < 0.055)) p.fast = false;
         }
     return p;
+}
+
+// PGW_FLAG_REINTERP: the column kernel, or (replay != null) its replay for iteration N
+int launch_reinterp(const pgw_timestep_args *a, const pgw_column_plan &plan, const pgw_timestep_result *replay,
+                    cudaStream_t st) {
+    auto kern = plan.fast ? pgw::pgw_column_kernel<kColumnThreads, true, false, false, true>
+                          : pgw::pgw_column_kernel<kColumnThreads, false, false, false, true>;
+    int rc = pgw_ensure_smem((const void *)kern, plan.fast ? 11 : 10, plan.smem, plan.np);
+    if (rc != PGW_OK) return rc;
+    const unsigned grid = (unsigned)((a->ncol + kColumnThreads - 1) / kColumnThreads);
+    kern<<<grid, kColumnThreads, plan.smem, st>>>(*a, plan.lst, plan.np, plan.ncand, replay);
+    return pgw_check_launch("pgw_column_kernel");
 }
 
 }  // namespace
@@ -917,6 +1073,7 @@ int pgw_timestep(const pgw_timestep_args *a, void *stream) {
     pgw::pgw_timestep_init_kernel<<<1, 64, 0, st>>>(a->maxerr, a->stats, a->err, a->first_k, a->poly_fallback);
     if (plan.tma) return pgw_launch_column_tma(a, plan, st);
 
+    if (plan.reinterp) return launch_reinterp(a, plan, nullptr, st);
     const int variant = plan.local ? (plan.fast ? 9 : 8) : plan.ref ? 2 : (plan.fast ? 1 : 0);
     auto kern = plan.local ? (plan.fast ? pgw::pgw_column_kernel<kColumnThreads, true, false, true>
                                         : pgw::pgw_column_kernel<kColumnThreads, false, false, true>)
@@ -925,7 +1082,7 @@ int pgw_timestep(const pgw_timestep_args *a, void *stream) {
                                         : pgw::pgw_column_kernel<kColumnThreads, false, false>);
     if ((rc = pgw_ensure_smem((const void *)kern, variant, plan.smem, plan.np)) != PGW_OK) return rc;
     const unsigned grid = (unsigned)((a->ncol + kColumnThreads - 1) / kColumnThreads);
-    kern<<<grid, kColumnThreads, plan.smem, st>>>(*a, plan.lst, plan.np, plan.ncand);
+    kern<<<grid, kColumnThreads, plan.smem, st>>>(*a, plan.lst, plan.np, plan.ncand, nullptr);
     return pgw_check_launch("pgw_column_kernel");
 }
 
@@ -934,6 +1091,12 @@ int pgw_timestep_finalize(const pgw_timestep_args *a, pgw_timestep_result *resul
     if (rc != PGW_OK || !result_dev) return PGW_E_INVALID;
     cudaStream_t st = (cudaStream_t)stream;
     pgw::pgw_converge_kernel<<<1, 1, 0, st>>>(a->maxerr, a->k_spec, a->thresh_phi_ref_max_error, result_dev);
+    // PGW_FLAG_REINTERP: the speculative QV does not give e_pgw of iteration N back (T and RELHUM move with the
+    // pressures), so the column kernel itself runs again for k_spec = N when the result was rewritten
+    if (a->flags & PGW_FLAG_REINTERP) {
+        if ((rc = launch_reinterp(a, plan_column(a), result_dev, st)) != PGW_OK) return rc;
+        return pgw_check_launch("pgw_timestep_finalize");
+    }
     const unsigned grid = (unsigned)((a->ncol + 255) / 256);
     pgw::pgw_rewrite_kernel<<<grid, 256, 0, st>>>(*a, result_dev);
     return pgw_check_launch("pgw_timestep_finalize");

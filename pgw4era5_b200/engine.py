@@ -324,9 +324,11 @@ class PGWEngine:
         T, QV, U, V [1,L,ny,nx] (the names of settings.var_name_map).  Returns a
         ``Pending``; nothing is synchronised here.
         """
-        if settings.i_reinterp or (settings.p_ref_inp is None and getattr(settings, "i_reference_dtypes", 0)):
-            raise ValueError("i_reinterp = 1 / p_ref_inp = None with i_reference_dtypes = 1 run through the "
-                             "staged path: use apply()")
+        ref_dtypes = getattr(settings, "i_reference_dtypes", 0)
+        if (settings.i_reinterp and settings.p_ref_inp is None) or \
+                ((settings.i_reinterp or settings.p_ref_inp is None) and ref_dtypes):
+            raise ValueError("i_reinterp = 1 with p_ref_inp = None, and either of them with i_reference_dtypes = 1, "
+                             "run through the staged path: use apply()")
         a, f, out, ws, k_spec, k_max = self._fill_args(era, era_step_dt, out, k_spec, slot)
         if direct:
             a.flags |= N.FLAG_DIRECT          # every parked level integrated in every iteration
@@ -463,6 +465,8 @@ class PGWEngine:
         a.k_spec = k_spec
         a.ps_bound = self.ps_bound
         a.flags = N.FLAG_REF_DTYPES if getattr(settings, "i_reference_dtypes", 0) else 0
+        if settings.i_reinterp:
+            a.flags |= N.FLAG_REINTERP        # re-interpolate the ERA state every iteration (step_03:202-216)
         if local:
             if self._zg_tables is None:
                 plev = np.ascontiguousarray(zg["plev"], dtype=np.float64)
@@ -553,9 +557,9 @@ class PGWEngine:
         return res
 
     def apply(self, era, era_step_dt, **kw):
-        """Synchronous form of ``submit``: returns the output dict (device tensors).  i_reinterp = 1,
-        which the fused pass does not cover, and p_ref_inp = None take the staged path (``submit``
-        runs p_ref_inp = None in the fused pass)."""
+        """Synchronous form of ``submit``: returns the output dict (device tensors).  i_reinterp = 1 and
+        p_ref_inp = None take the staged path (``submit`` runs each of them, though not both together, in
+        the fused pass)."""
         if settings.i_reinterp or settings.p_ref_inp is None:
             from . import staged
             kw.pop("k_spec", None)

@@ -63,7 +63,7 @@ p_ref_inp = 30000  # Pa; None = choose locally (PGWEngine.submit: fused kernel; 
 adj_factor = 0.95
 thresh_phi_ref_max_error = 0.15
 max_n_iter = 20
-i_reinterp = 0
+i_reinterp = 0     # 1: re-interpolate the ERA state every iteration (PGWEngine.submit: fused kernel; apply: staged path)
 
 # Not in the reference's settings.py.  The reference never casts, so what it computes in follows from the
 # dtypes of the ERA5 file: with float32 PS and FIS (every real file) delta_ps / ps_pgw are float32 and the
