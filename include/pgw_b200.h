@@ -27,10 +27,11 @@
 extern "C" {
 #endif
 
-#define PGW_B200_ABI_VERSION 8   /* 6: + pgw_timestep_status, pgw_timestep_run/_finish, PGW_FLAG_REF_DTYPES, first_k,
+#define PGW_B200_ABI_VERSION 9   /* 6: + pgw_timestep_status, pgw_timestep_run/_finish, PGW_FLAG_REF_DTYPES, first_k,
                                        pgw_band_pack/_unpack, pgw_band_exchange, pgw_regrid_bilinear_band_f32
                                     7: + PGW_FLAG_LOCAL_PREF and its args, PGW_ERR_PREF_FLOOR, first_k[4]
-                                    8: + PGW_FLAG_REINTERP (no layout change) */
+                                    8: + PGW_FLAG_REINTERP (no layout change)
+                                    9: + pgw_pack_d4_f32 */
 
 /* host-side return codes */
 #define PGW_OK               0
@@ -456,6 +457,16 @@ int pgw_gauss_interp_f64(const double *src_lat_m, const double *src_lon_m, const
  * inside open_dataset / to_netcdf (step_03_apply_to_era.py:60, :378) for the float32 fields.
  * ---------------------------------------------------------------------- */
 int pgw_byteswap32(void *data, long long n, void *stream);
+
+/* ------------------------------------------------------------------------
+ * Streamed climatology: one delta stamp of ta, hur, ua, va (n = K*ncol 32-bit words each) into the
+ * node layout of the column kernel, out[i] = {ta[i], hur[i], ua[i], va[i]} (out: float4[n], 16-byte
+ * aligned).  swap = 1 also reverses the byte order of every word (raw NetCDF-3 records are big-endian).
+ * Words are moved, not converted: NaN payloads survive.  Any n and any 4-byte alignment of the inputs;
+ * 16-byte loads when all four are 16-byte aligned.
+ * ---------------------------------------------------------------------- */
+int pgw_pack_d4_f32(const void *ta, const void *hur, const void *ua, const void *va, void *out, long long n,
+                    int swap, void *stream);
 
 #ifdef __cplusplus
 }

@@ -73,7 +73,7 @@ class TimestepStatus(C.Structure):
                 ("err", C.c_uint32), ("first_k", C.c_int32 * 4), ("poly_fallback", C.c_uint32)]
 
 
-ABI_VERSION = 8          # PGW_B200_ABI_VERSION of include/pgw_b200.h
+ABI_VERSION = 9         # PGW_B200_ABI_VERSION of include/pgw_b200.h
 
 
 class NativeError(RuntimeError):
@@ -109,6 +109,7 @@ def _load():
         "pgw_integrate_tos_f64": (i, [vp, vp, vp, vp, vp, ll, vp]),
         "pgw_time_interp_f32": (i, [vp, vp, d, d, vp, ll, vp]),
         "pgw_byteswap32": (i, [vp, ll, vp]),
+        "pgw_pack_d4_f32": (i, [vp, vp, vp, vp, vp, ll, i, vp]),
         "pgw_geod_to_meter_f64": (i, [vp, vp, vp, vp, vp, ll, vp]),
         "pgw_gauss_interp_f64": (i, [vp, vp, vp, ll, i, vp, vp, vp, vp, ll, d, d, vp]),
         "pgw_time_mean_f32": (i, [vp, i, vp, ll, vp]),

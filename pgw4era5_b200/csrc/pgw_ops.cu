@@ -369,6 +369,49 @@ int pgw_byteswap32(void *data, long long n, void *stream) {
     return pgw_check_launch("byteswap32_kernel");
 }
 
+// ---------------------------------------------------------------------------
+// One stamp of ta, hur, ua, va into the engine's node layout d4 (one float4 per pressure node and column),
+// optionally swapping the byte order of big-endian NetCDF-3 records on the way.  Words are moved, never
+// converted, so NaN payloads survive.  A thread packs four consecutive nodes from one 16-byte load per input
+// when every input is 16-byte aligned; otherwise (and for the last n % 4 nodes) one node per word load.
+// ---------------------------------------------------------------------------
+namespace pgw {
+__device__ __forceinline__ uint32_t maybe_swap(uint32_t x, int swap) { return swap ? __byte_perm(x, 0, 0x0123) : x; }
+
+__global__ void __launch_bounds__(256) pack_d4_kernel(const uint32_t *__restrict__ a, const uint32_t *__restrict__ b,
+                                                     const uint32_t *__restrict__ c, const uint32_t *__restrict__ d,
+                                                     uint4 *__restrict__ out, long long n, int swap, int vec) {
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    const long long t0 = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const long long n4 = vec ? n >> 2 : 0;
+    for (long long i = t0; i < n4; i += stride) {
+        const uint4 x = reinterpret_cast<const uint4 *>(a)[i], y = reinterpret_cast<const uint4 *>(b)[i];
+        const uint4 z = reinterpret_cast<const uint4 *>(c)[i], w = reinterpret_cast<const uint4 *>(d)[i];
+        uint4 *o = out + 4 * i;
+        o[0] = make_uint4(maybe_swap(x.x, swap), maybe_swap(y.x, swap), maybe_swap(z.x, swap), maybe_swap(w.x, swap));
+        o[1] = make_uint4(maybe_swap(x.y, swap), maybe_swap(y.y, swap), maybe_swap(z.y, swap), maybe_swap(w.y, swap));
+        o[2] = make_uint4(maybe_swap(x.z, swap), maybe_swap(y.z, swap), maybe_swap(z.z, swap), maybe_swap(w.z, swap));
+        o[3] = make_uint4(maybe_swap(x.w, swap), maybe_swap(y.w, swap), maybe_swap(z.w, swap), maybe_swap(w.w, swap));
+    }
+    for (long long i = (n4 << 2) + t0; i < n; i += stride)
+        out[i] = make_uint4(maybe_swap(a[i], swap), maybe_swap(b[i], swap), maybe_swap(c[i], swap),
+                            maybe_swap(d[i], swap));
+}
+}  // namespace pgw
+
+int pgw_pack_d4_f32(const void *ta, const void *hur, const void *ua, const void *va, void *out, long long n,
+                    int swap, void *stream) {
+    PGW_REQUIRE(ta && hur && ua && va && out && n > 0 && (swap == 0 || swap == 1));
+    PGW_REQUIRE((reinterpret_cast<uintptr_t>(out) & 15u) == 0);
+    const uintptr_t any = reinterpret_cast<uintptr_t>(ta) | reinterpret_cast<uintptr_t>(hur) |
+                          reinterpret_cast<uintptr_t>(ua) | reinterpret_cast<uintptr_t>(va);
+    const int vec = (any & 15u) == 0;
+    pgw::pack_d4_kernel<<<ew_grid(vec ? (n + 3) / 4 : n, 256), 256, 0, (cudaStream_t)stream>>>(
+        static_cast<const uint32_t *>(ta), static_cast<const uint32_t *>(hur), static_cast<const uint32_t *>(ua),
+        static_cast<const uint32_t *>(va), static_cast<uint4 *>(out), n, swap, vec);
+    return pgw_check_launch("pack_d4_kernel");
+}
+
 int pgw_time_mean_f32(const float *series, int ntime, float *out, long long n, void *stream) {
     PGW_REQUIRE(series && out && ntime > 0 && n > 0);
     time_mean_kernel<<<ew_grid(n, 256), 256, 0, (cudaStream_t)stream>>>(series, ntime, out, n);

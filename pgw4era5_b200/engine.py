@@ -47,41 +47,21 @@ def _stream():
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
-class DeltaSet:
-    """
-    Climate deltas resident on one GPU.
+def read_axes(name, d):
+    """(kept stamps, indices of the kept stamps in the source, plev or None) of one delta variable in the dict
+    form ``DeltaSet`` takes; 29 February is dropped (functions.py:224-230)."""
+    stamps = np.asarray(d["time"]).astype("datetime64[ns]")
+    keep = timeinterp.drop_leap_day(stamps)
+    plev = None if d.get("plev") is None else np.asarray(d["plev"], dtype=np.float64)
+    return stamps[keep], keep, plev
 
-    ``deltas``: var -> dict(time=datetime64[nt], plev=[K] or None, data=[nt,(K),ny,nx])
-    for ta, hur, ua, va, zg, tas, hurs, ts, tos, siconc (SCEN-HIST) and ``ps_hist``
-    (the HIST ps climatology, functions.py:330-332).  29 February is dropped
-    once here (functions.py:224-230).
 
-    Layout in HBM: ta, hur, ua, va are interleaved per pressure node and column as
-    ``d4[nt, K, ny, nx, 4]`` (one 16-byte load per node, month and column in the column
-    kernel); ``vars[name]["data"]`` of these four are strided views of ``d4``.  zg and
-    the 2-D deltas stay separate, contiguous fields.
-    """
+class DeltaSetBase:
+    """What the resident and the streamed delta set share: the pressure axis of the packed deltas and its checks,
+    which two stamps bracket an ERA5 date, the slabs of resident variables and ``ts_clim``.  Subclasses fill
+    ``vars`` (name -> dict(time, plev, data)) and call ``_check_axes`` with the shapes of ta, hur, ua, va."""
 
-    def __init__(self, deltas, device="cuda"):
-        self.device = torch.device(device)
-        self.vars = {}
-        staged = {}
-        for name in VARS_3D + VARS_2D:
-            if name not in deltas:
-                raise KeyError("climate delta %r missing" % name)
-            d = deltas[name]
-            stamps = np.asarray(d["time"]).astype("datetime64[ns]")
-            keep = timeinterp.drop_leap_day(stamps)
-            data = d["data"]
-            if not isinstance(data, torch.Tensor):
-                data = torch.as_tensor(np.asarray(data))
-            if len(keep) != len(stamps):
-                data = data[torch.as_tensor(keep, device=data.device)]
-            plev = None if d.get("plev") is None else np.asarray(d["plev"], dtype=np.float64)
-            self.vars[name] = dict(time=stamps[keep], plev=plev, data=None)
-            staged[name] = data
-        self.shape2d = tuple(staged["ts"].shape[-2:])
-        self.ncol = self.shape2d[0] * self.shape2d[1]
+    def _check_axes(self, shapes):
         plev = self.vars["ta"]["plev"]
         for name in ("hur", "ua", "va"):
             if not np.array_equal(self.vars[name]["plev"], plev):
@@ -97,29 +77,9 @@ class DeltaSet:
         for name in ("hur", "ua", "va"):
             if not np.array_equal(self.vars[name]["time"], stamps):
                 raise ValueError("ta, hur, ua, va deltas must share their time stamps")
-            if tuple(staged[name].shape) != tuple(staged["ta"].shape):
+            if tuple(shapes[name]) != tuple(shapes["ta"]):
                 raise ValueError("ta, hur, ua, va deltas must share their shape")
-        # ONE arena holds the whole climatology (the packed float4 nodes first: 16-byte aligned), so that
-        # replicating it to the other GPUs is one NCCL broadcast (parallel.broadcast_deltas)
-        shapes = [("d4", tuple(staged["ta"].shape) + (4,))] + \
-                 [(n, tuple(staged[n].shape)) for n in ("zg",) + VARS_2D]
-        offs, total = {}, 0
-        for name, shp in shapes:
-            offs[name] = total
-            total += (int(np.prod(shp)) + 3) // 4 * 4
-        self.arena = torch.empty(total, device=self.device, dtype=torch.float32)
-        view = lambda name, shp: self.arena[offs[name]:offs[name] + int(np.prod(shp))].view(shp)
-        self.d4 = view(*shapes[0])
-        for i, name in enumerate(VARS_PACKED):
-            self.d4[..., i].copy_(staged.pop(name).to(self.device, torch.float32))
-            self.vars[name]["data"] = self.d4[..., i]
-        for name, shp in shapes[1:]:
-            v = view(name, shp)
-            v.copy_(staged.pop(name).to(self.device, torch.float32))
-            self.vars[name]["data"] = v
         self._brackets, self._moved, self._time_group, self._time_ids, self._lay = {}, {}, {}, {}, {}
-        self.ts_clim = None
-        self.refresh_derived()
 
     def refresh_derived(self):
         """Annual mean of the ts delta (step_03_apply_to_era.py:134-136), computed once."""
@@ -130,10 +90,6 @@ class DeltaSet:
                 "pgw_time_mean_f32")
         # the pipelines run on their own streams, which do not wait for the stream the arena was filled on
         torch.cuda.current_stream().synchronize()
-
-    def tensors(self):
-        """The device memory that holds the climatology (for the NCCL broadcast): one arena."""
-        return [self.arena]
 
     def bracket(self, name, when):
         """TimeBracket of variable ``name`` for the ERA5 date ``when``; variables that share their time axis
@@ -174,6 +130,74 @@ class DeltaSet:
         off = base + (sl * level if level is not None else 0)
         nt = len(self.vars[name]["time"])
         return N.TSlab(off + st * (b.ind_before % nt), off + st * (b.ind_after % nt), b.x_hi, b.x_new)
+
+
+class DeltaSet(DeltaSetBase):
+    """
+    Climate deltas resident on one GPU.
+
+    ``deltas``: var -> dict(time=datetime64[nt], plev=[K] or None, data=[nt,(K),ny,nx])
+    for ta, hur, ua, va, zg, tas, hurs, ts, tos, siconc (SCEN-HIST) and ``ps_hist``
+    (the HIST ps climatology, functions.py:330-332).  29 February is dropped
+    once here (functions.py:224-230).
+
+    Layout in HBM: ta, hur, ua, va are interleaved per pressure node and column as
+    ``d4[nt, K, ny, nx, 4]`` (one 16-byte load per node, month and column in the column
+    kernel); ``vars[name]["data"]`` of these four are strided views of ``d4``.  zg and
+    the 2-D deltas stay separate, contiguous fields.
+    """
+
+    def __init__(self, deltas, device="cuda"):
+        self.device = torch.device(device)
+        self.vars = {}
+        staged = {}
+        for name in VARS_3D + VARS_2D:
+            if name not in deltas:
+                raise KeyError("climate delta %r missing" % name)
+            d = deltas[name]
+            stamps, keep, plev = read_axes(name, d)
+            data = d["data"]
+            if not isinstance(data, torch.Tensor):
+                data = torch.as_tensor(np.asarray(data))
+            if len(keep) != len(d["time"]):
+                data = data[torch.as_tensor(keep, device=data.device)]
+            self.vars[name] = dict(time=stamps, plev=plev, data=None)
+            staged[name] = data
+        self.shape2d = tuple(staged["ts"].shape[-2:])
+        self.ncol = self.shape2d[0] * self.shape2d[1]
+        self._check_axes({name: staged[name].shape for name in VARS_PACKED})
+        # ONE arena holds the whole climatology (the packed float4 nodes first: 16-byte aligned), so that
+        # replicating it to the other GPUs is one NCCL broadcast (parallel.broadcast_deltas)
+        shapes = [("d4", tuple(staged["ta"].shape) + (4,))] + \
+                 [(n, tuple(staged[n].shape)) for n in ("zg",) + VARS_2D]
+        offs, total = {}, 0
+        for name, shp in shapes:
+            offs[name] = total
+            total += (int(np.prod(shp)) + 3) // 4 * 4
+        self.arena = torch.empty(total, device=self.device, dtype=torch.float32)
+        view = lambda name, shp: self.arena[offs[name]:offs[name] + int(np.prod(shp))].view(shp)
+        self.d4 = view(*shapes[0])
+        for i, name in enumerate(VARS_PACKED):
+            self.d4[..., i].copy_(staged.pop(name).to(self.device, torch.float32))
+            self.vars[name]["data"] = self.d4[..., i]
+        for name, shp in shapes[1:]:
+            v = view(name, shp)
+            v.copy_(staged.pop(name).to(self.device, torch.float32))
+            self.vars[name]["data"] = v
+        self.ts_clim = None
+        self.refresh_derived()
+
+    def tensors(self):
+        """The device memory that holds the climatology (for the NCCL broadcast): one arena."""
+        return [self.arena]
+
+    def hold(self, stream=None):
+        """The stamps handed out since the last call stay in use until ``stream`` gets here.  Every stamp is
+        resident, so there is nothing to record."""
+
+    def stamp(self, name, i):
+        """Kept stamp ``i`` of variable ``name`` as a device tensor ([K, ny, nx] or [ny, nx])."""
+        return self.vars[name]["data"][i]
 
     def slab4(self, when):
         """pgw_tslab of the packed (ta, hur, ua, va) deltas at ERA5 time ``when``."""
@@ -244,6 +268,8 @@ class PGWEngine:
         self.p_floor = float(p_floor)
         self._zg_tables = None
         self.group = group
+        if group is not None and getattr(deltas, "streamed", False):
+            raise ValueError("latitude bands need a resident DeltaSet: a streamed delta set is not supported")
         # latitude-band mode: how the bands agree on the iteration count.  "p2p": pgw_band_exchange, one kernel over
         # peer memory behind the column kernel (inboxes in torch symmetric memory); "nccl": pack, all-reduce(MAX),
         # unpack; "auto": p2p where the peer mapping can be set up, else nccl.
@@ -365,6 +391,7 @@ class PGWEngine:
             N.check(N.lib.pgw_timestep_finish(C.byref(a), sdev, shost, st), "pgw_timestep_finish")
         self.stats["launches"] += 4
         ws["event"].record()
+        self.deltas.hold(torch.cuda.current_stream())      # a streamed set keeps this timestep's stamps until here
         ctx = dict(era=era, when=era_step_dt, ignore_top=ignore_top_pressure_error, k_spec=k_spec,
                    k_max=k_max, keep=(f, a), file_name=file_name, slot=slot, direct=direct,
                    stream=torch.cuda.current_stream(), local_pref=bool(a.flags & N.FLAG_LOCAL_PREF))

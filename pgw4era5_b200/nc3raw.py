@@ -199,6 +199,24 @@ class RawNC3:
                 raise IOError("unexpected end of %s while reading %s" % (self.path, name))
             done += n
 
+    def read_stamp(self, fobj, name, buf, i):
+        """Raw big-endian bytes of entry ``i`` of the first axis of ``name`` into ``buf``: record ``i`` of a
+        record variable, else the slice at ``begin + i * bytes per entry``."""
+        v = self.vars[name]
+        if v.is_record:
+            return self.read_into(fobj, name, buf, record=i)
+        mv = memoryview(buf).cast("B")
+        step = int(np.prod(v.shape[1:], dtype=np.int64)) * v.dtype.itemsize
+        if mv.nbytes != step or not 0 <= i < v.shape[0]:
+            raise ValueError("%s: entry %d of %d, buffer has %d bytes, entry %d" % (name, i, v.shape[0], mv.nbytes,
+                                                                                  step))
+        off, done = v.begin + i * step, 0
+        while done < mv.nbytes:
+            n = os.preadv(fobj.fileno(), [mv[done:]], off + done)
+            if n <= 0:
+                raise IOError("unexpected end of %s while reading %s" % (self.path, name))
+            done += n
+
     def write_from(self, fd, name, buf, record=0):
         """Overwrite the values of ``name`` in the file open as descriptor ``fd`` with raw big-endian bytes."""
         v = self.vars[name]

@@ -51,6 +51,8 @@ def broadcast_deltas(deltas, src=0, group=None, info=None):
     the elapsed ms of the broadcast itself; ``info`` (a dict) also receives bytes and GB/s."""
     import torch
     import torch.distributed as dist
+    if getattr(deltas, "streamed", False):
+        raise ValueError("a streamed delta set cannot be broadcast: every rank reads the delta files itself")
     warm = torch.zeros(1, device=deltas.device)
     dist.broadcast(warm, src=src, group=group)
     torch.cuda.synchronize()

@@ -54,8 +54,7 @@ def _blend(ds, name, when, level=None):
     """load_delta's two-point time interpolation (functions.py:288-292) of one resident delta:
     float64 arithmetic, float32 storage (pgw_time_interp_f32), returned as float64."""
     b = ds.bracket(name, when)
-    data = ds.vars[name]["data"]
-    lo, hi = data[b.ind_before], data[b.ind_after]
+    lo, hi = ds.stamp(name, b.ind_before), ds.stamp(name, b.ind_after)
     if level is not None:
         lo, hi = lo[level], hi[level]
     lo, hi = lo.contiguous(), hi.contiguous()
@@ -68,6 +67,13 @@ def _blend(ds, name, when, level=None):
 def apply_staged(eng, era, era_step_dt, out=None, ignore_top_pressure_error=False, file_name="<memory>"):
     """One ERA5 timestep through the staged path.  Same inputs and outputs as ``PGWEngine.apply``;
     with ``p_ref_inp = None`` the result also carries ``p_ref`` [1, ny, nx]."""
+    try:
+        return _apply_staged(eng, era, era_step_dt, out, ignore_top_pressure_error, file_name)
+    finally:                                         # a streamed delta set keeps the stamps read here until then
+        eng.deltas.hold(torch.cuda.current_stream())
+
+
+def _apply_staged(eng, era, era_step_dt, out, ignore_top_pressure_error, file_name):
     ds = eng.deltas
     a, f, out, ws, _, _ = eng._fill_args(era, era_step_dt, out, k_spec=1)
     ny, nx = f["PS"].shape[-2:]

@@ -25,15 +25,21 @@ from .parallel import IterMP
 _ENGINES = {}
 
 
-def load_delta_set(delta_input_dir, device="cuda"):
+def load_delta_set(delta_input_dir, device="cuda", max_resident_bytes=None):
     """Read every delta file the path needs (ta, hur, ua, va, zg, tas, hurs, ts, tos, siconc as
-    SCEN-HIST, ps as HIST; step_03_apply_to_era.py:533-539) into one device-resident DeltaSet."""
+    SCEN-HIST, ps as HIST; step_03_apply_to_era.py:533-539) into one device-resident DeltaSet, or, when
+    that set and the staging copy of one variable would take more than ``max_resident_bytes`` (default:
+    half of the device's free memory), into a ``StreamedDeltaSet`` that reads the 3-D deltas of NetCDF-3
+    files stamp by stamp.  Only the headers and coordinates of the 3-D files are read to decide."""
+    from . import deltastream
     from .engine import DeltaSet, VARS_2D, VARS_3D
+    headers = deltastream.read_3d_headers(delta_input_dir)
+    if deltastream.should_stream(headers, device, max_resident_bytes):
+        return deltastream.open_streamed(delta_input_dir, headers, device=device)
     deltas = {}
     for name in VARS_3D + VARS_2D:
-        var_name, base = ("ps", settings.file_name_bases['HIST']) if name == "ps_hist" else \
-            (name, settings.file_name_bases['SCEN-HIST'])
-        ds = ncio.open_dataset(os.path.join(delta_input_dir, base.format(var_name)))
+        path, var_name = deltastream.delta_file(delta_input_dir, name)
+        ds = ncio.open_dataset(path)
         var = ds[var_name]
         plev = None
         if settings.PLEV_GCM in var.dims:
