@@ -314,6 +314,10 @@ long long pgw_timestep_smem_bytes(const pgw_timestep_args *a);
  * PGW_FLAG_REF_DTYPES, and PGW_FLAG_LOCAL_PREF and PGW_FLAG_REINTERP on every grid: the TMA flavour handles a
  * scalar p_ref and iteration-invariant parked levels only) */
 int pgw_timestep_uses_tma(const pgw_timestep_args *a);
+/* Resources per CTA of the TMA flavour for nplev pressure nodes, nlev levels and np parked levels (even): the
+ * tensor-memory columns it allocates and the bytes of dynamic shared memory it is launched with (padded to the
+ * CTA's share of the SM's tensor memory).  Host arithmetic only; PGW_E_INVALID for arguments out of range. */
+int pgw_column_tma_layout(int nplev, int nlev, int np, int *tmem_cols, long long *smem_bytes);
 int pgw_timestep(const pgw_timestep_args *a, void *stream);
 
 /* device-side result of the convergence scan, written by finalize */

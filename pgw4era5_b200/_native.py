@@ -115,6 +115,7 @@ def _load():
         "pgw_time_mean_f32": (i, [vp, i, vp, ll, vp]),
         "pgw_timestep_smem_bytes": (ll, [C.POINTER(TimestepArgs)]),
         "pgw_timestep_uses_tma": (i, [C.POINTER(TimestepArgs)]),
+        "pgw_column_tma_layout": (i, [i, i, i, C.POINTER(C.c_int), C.POINTER(C.c_longlong)]),
         "pgw_timestep": (i, [C.POINTER(TimestepArgs), vp]),
         "pgw_timestep_finalize": (i, [C.POINTER(TimestepArgs), vp, vp]),
         "pgw_sizeof_timestep_status": (ll, []),

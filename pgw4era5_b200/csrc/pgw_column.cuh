@@ -301,6 +301,62 @@ template <int N>
 __device__ __forceinline__ void tma_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
 __device__ __forceinline__ void tma_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 
+// ---------------------------------------------------------------------------
+// Register reallocation between warpgroups and tensor memory (tcgen05, sm_100a)
+// ---------------------------------------------------------------------------
+// setmaxnreg: every warp of the warpgroup must execute the same instruction
+template <int N>
+__device__ __forceinline__ void regs_dec() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(N)); }
+template <int N>
+__device__ __forceinline__ void regs_inc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(N)); }
+// One warp allocates `ncols` (a power of two >= 32) columns of all 128 lanes and writes the address to shared
+// memory; relinquishing the permit lets a co-resident CTA allocate without waiting for this one to exit.
+__device__ __forceinline__ void tmem_alloc(uint32_t *dst, uint32_t ncols) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst)), "r"(ncols)
+                 : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+}
+// order tcgen05 operations around a thread synchronisation (barrier) of the CTA
+__device__ __forceinline__ void tmem_fence_before_sync() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void tmem_fence_after_sync() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+// A warp reaches the 32 lanes 32 (warp % 4) .. +31; taddr = (lane << 16) | column, warp-uniform.
+// 32x32b shape: lane i of the warp stores / loads TMEM lane (base + i), consecutive columns.
+__device__ __forceinline__ void tmem_st4(uint32_t taddr, float a, float b, float c, float d) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};" ::"r"(taddr), "r"(__float_as_uint(a)),
+                 "r"(__float_as_uint(b)), "r"(__float_as_uint(c)), "r"(__float_as_uint(d)) : "memory");
+}
+__device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+// loads end in tcgen05.wait::ld inside the same asm statement, so no use of the values can move above it
+__device__ __forceinline__ float2 tmem_ld2(uint32_t taddr) {
+    uint32_t x, y;
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x2.b32 {%0, %1}, [%2];\n\t"
+                 "tcgen05.wait::ld.sync.aligned;" : "=r"(x), "=r"(y) : "r"(taddr) : "memory");
+    return make_float2(__uint_as_float(x), __uint_as_float(y));
+}
+__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8]) {
+    uint32_t r[8];
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];\n\t"
+                 "tcgen05.wait::ld.sync.aligned;"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
+                 : "r"(taddr) : "memory");
+#pragma unroll
+    for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
+}
+__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
+    uint32_t r[16];
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, "
+                 "%14, %15}, [%16];\n\t"
+                 "tcgen05.wait::ld.sync.aligned;"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
+                   "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+                 : "r"(taddr) : "memory");
+#pragma unroll
+    for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
+}
+
 }  // namespace pgw
 
 // ---- host-side pieces shared by pgw_timestep.cu and pgw_column_tma.cu

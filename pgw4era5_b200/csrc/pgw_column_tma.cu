@@ -2,12 +2,17 @@
 //
 // Same algorithm and reference semantics as pgw_timestep.cu (see the header comment there):
 // one thread owns one ERA5 column, the column is swept bottom-up, the levels below p_ref are
-// parked in shared memory for the surface-pressure fixed point, the rest is streamed with the
-// adjusted surface pressure already known.  What differs is how the 3-D fields move:
+// parked for the surface-pressure fixed point, the rest is streamed with the adjusted surface
+// pressure already known.  What differs is how the 3-D fields move and where the parked levels live:
 //
-//  * a fifth warp (one elected thread) streams level PAIRS of the CTA's 128 columns through a
-//    ring of shared-memory slots [T,QV,U,V][2 levels][128] with cp.async.bulk.tensor (TMA,
-//    box 2 x 128 of a [nlev, ncol] tensor map per field);
+//  * the CTA is two warpgroups.  The first (producer) gives its registers to the second with
+//    setmaxnreg (64 at launch -> 24 / 104), so 4 CTAs = 16 column warps fit on an SM, and one
+//    elected thread of it streams level PAIRS of the CTA's 128 columns through a ring of
+//    shared-memory slots [T,QV,U,V][2 levels][128] with cp.async.bulk.tensor (TMA, box 2 x 128 of a
+//    [nlev, ncol] tensor map per field);
+//  * the second warpgroup holds the four column warps; column thread i parks (T_pgw, e_pgw) of its
+//    levels in TENSOR MEMORY lane i (tcgen05.st / tcgen05.ld), which leaves shared memory to the ring
+//    and the tables;
 //  * the four column warps wait on full[slot], read their column from the slot, compute, write
 //    the results back IN PLACE, fence them for the async proxy and arrive on done[slot];
 //  * the producer then stores the slot with TMA (bulk group), and, once the previous slot's
@@ -87,19 +92,21 @@ __device__ __forceinline__ F4 ldg4(const float4 *p) { const float4 v = __ldg(p);
 // arguments).  The loop bounds of the sweep are then immediates; with run-time bounds every pair iteration
 // waits on a constant-bank load before it can resolve its branches.  The host picks the instance that
 // matches (137 levels with 56 parked ones: ERA5 L137, p_ref = 300 hPa) or the generic one.
+//
+// Tensor memory: `ncols` columns (host: next power of two >= max(32, 2 np)); parked level l sits in columns
+// 2 (L-1-l) (T_pgw) and 2 (L-1-l) + 1 (e_pgw), so a parked level pair is one 4-column store.
 template <bool FAST, int NLEV_C, int NP_C>
-__global__ void __launch_bounds__(kColumnThreads + 32, 3)
+__global__ void __launch_bounds__(2 * kColumnThreads, 4)
 pgw_column_tma_kernel(const __grid_constant__ pgw_timestep_args a, const __grid_constant__ TmaParams tp,
-                      const int lst_arg, const int np_arg) {
-    constexpr int NT = kColumnThreads;
+                      const int lst_arg, const int np_arg, const uint32_t ncols) {
+    constexpr int NT = kColumnThreads, NTHR = 2 * kColumnThreads;
     extern __shared__ __align__(1024) unsigned char smem[];
     const int L = NLEV_C ? NLEV_C : a.nlev, K = a.nplev;
     const int np = NP_C ? NP_C : np_arg;
     const int lst = NLEV_C ? NLEV_C - NP_C : lst_arg;
-    // ---- shared memory: pair ring | stash | (ak,bk)[np+1] | (akm,bkm)[np] | plev tables | barriers
+    // ---- shared memory: pair ring | (ak,bk)[np+1] | (akm,bkm)[np] | plev tables | barriers | TMEM address
     float *const ring = reinterpret_cast<float *>(smem);                          // [kTmaSlots][4][2][NT]
-    float2 *const st_Te = reinterpret_cast<float2 *>(ring + kTmaSlots * 8 * NT);    // [np][NT] (T_pgw fp32, e_pgw)
-    double2 *const hl0 = reinterpret_cast<double2 *>(st_Te + (size_t)np * NT);
+    double2 *const hl0 = reinterpret_cast<double2 *>(ring + kTmaSlots * 8 * NT);
     float2 *const m0p = reinterpret_cast<float2 *>(hl0 + (np + 1));
     float *const s_plev = reinterpret_cast<float *>(m0p + np);                     // [K] ascending
     float *const s_inv_plev = s_plev + K;                                          // [K]
@@ -113,13 +120,15 @@ pgw_column_tma_kernel(const __grid_constant__ pgw_timestep_args a, const __grid_
     uint64_t *const bar_full = reinterpret_cast<uint64_t *>(s_plev + 3 * K + ((3 * K) & 1));
 #endif
     uint64_t *const bar_done = bar_full + kTmaSlots;
+    uint32_t *const s_tmem = reinterpret_cast<uint32_t *>(bar_done + kTmaSlots);
+    int *const s_lstar = reinterpret_cast<int *>(s_tmem + 1);                     // [NT]
     const double2 *const s_hl = hl0 - lst;      // indexed by the half level, l >= lst
     const float2 *const s_m = m0p - lst;        // indexed by the full level, l >= lst
 
     const int tid = threadIdx.x;
-    for (int i = tid; i <= np; i += NT + 32) hl0[i] = make_double2(a.ak[lst + i], a.bk[lst + i]);
-    for (int i = tid; i < np; i += NT + 32) m0p[i] = make_float2((float)a.akm[lst + i], (float)a.bkm[lst + i]);
-    for (int i = tid; i < K; i += NT + 32) {
+    for (int i = tid; i <= np; i += NTHR) hl0[i] = make_double2(a.ak[lst + i], a.bk[lst + i]);
+    for (int i = tid; i < np; i += NTHR) m0p[i] = make_float2((float)a.akm[lst + i], (float)a.bkm[lst + i]);
+    for (int i = tid; i < K; i += NTHR) {
         const int f0 = a.plev_descending ? (K - 1 - i) : i;
         const float p0 = (float)a.plev[f0];
         s_plev[i] = p0;
@@ -133,10 +142,13 @@ pgw_column_tma_kernel(const __grid_constant__ pgw_timestep_args a, const __grid_
         for (int i = 0; i < kTmaSlots; ++i) { mbar_init(bar_full + i, 1); mbar_init(bar_done + i, NT); }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
+    if ((tid >> 5) == NT / 32) tmem_alloc(s_tmem, ncols);        // the first column warp
+    tmem_fence_before_sync();
     __syncthreads();
+    tmem_fence_after_sync();
 #if PGW_UNIFORM_TOP
     // walker position and weight of the levels whose pressure is akm alone, by the instructions of walk()
-    for (int l = tid; l < L; l += NT + 32) {
+    for (int l = tid; l < L; l += NTHR) {
         const float2 m = tp.m[l];
         int nd = -1;
         for (int k = K - 1; k >= 0; --k)
@@ -150,9 +162,10 @@ pgw_column_tma_kernel(const __grid_constant__ pgw_timestep_args a, const __grid_
     const uint32_t n = (uint32_t)a.ncol;
     const int npairs = (L + 1) >> 1, np1 = np >> 1;     // level pairs in total / parked (np is even)
 
-    // ------------------------------------------------------------------ producer warp
-    if (tid >= NT) {
-        if (tid != NT) return;
+    // ------------------------------------------------------------------ producer warpgroup
+    if (tid < NT) {
+        regs_dec<24>();                                     // all four warps, before any of them exits
+        if (tid != 0) return;
         const int c0 = (int)(blockIdx.x * NT);
         // pair j = levels L-1-2j (row 1) and L-2-2j (row 0).  TMA coordinates must not be negative,
         // so the last pair of an odd column is levels (1, 0): level 1 is simply done twice.
@@ -192,7 +205,10 @@ pgw_column_tma_kernel(const __grid_constant__ pgw_timestep_args a, const __grid_
     }
 
     // ------------------------------------------------------------------ column threads
-    const uint32_t c_raw = blockIdx.x * NT + tid;
+    regs_inc<104>();
+    const int ct = tid - NT;                                // column of the CTA = TMEM lane
+    const uint32_t tm = *s_tmem + ((uint32_t)(ct & ~31) << 16);   // column 0 of this warp's 32 lanes
+    const uint32_t c_raw = blockIdx.x * NT + ct;
     // Threads past the last column read column n-1 for the 2-D fields; their slot columns are
     // zero-filled by TMA and clipped on store, and their per-thread stores are masked.
     const uint32_t c = (c_raw >= n) ? n - 1 : c_raw;
@@ -429,7 +445,7 @@ pgw_column_tma_kernel(const __grid_constant__ pgw_timestep_args a, const __grid_
 
     // ---------------- the geopotential sums of the parked levels ----------------
     // The fixed point needs phi(p_ref) of the PGW state for ps = PS + x, x = dps_k.  (T, e) of the parked
-    // levels are kept in shared memory, but instead of re-integrating all of them in every iteration, the
+    // levels are kept in tensor memory, but instead of re-integrating all of them in every iteration, the
     // sum over the layers that lie safely below p_ref is expanded ONCE, during the sweep, as a polynomial
     // in x:
     //   ln(P_h + b_h x) = ln P_h + u x - (u x)^2/2 + (u x)^3/3 - (u x)^4/4,  u = b_h / P_h <= 1/PS,
@@ -444,7 +460,9 @@ pgw_column_tma_kernel(const __grid_constant__ pgw_timestep_args a, const __grid_
     double acc_res = 0.0, acc_T0 = 0.0, acc_part0 = 0.0, t_low_d = 0.0;
     double S1 = 0.0, S2 = 0.0, S3 = 0.0, S4 = 0.0;            // sum_l T_l (ub^k - ut^k)
     float H1 = 0.0f, H2 = 0.0f, H3 = 0.0f;                    // humidity part, coefficients of x, x^2, x^3
-    int lstar = -1;                                           // the layer that contains p_ref for x = 0
+    // the layer that contains p_ref for x = 0 (-1: none).  Written once, in shared memory: a register for it across
+    // the parked pairs costs a spill there.
+    s_lstar[ct] = -1;
     auto rcp64 = [](double v) { double r = rcp64_approx(v); return fma(r, fma(-v, r, 1.0), r); };
     // add sgn * (contribution of the fully-below layer l) to the polynomial
     auto taylor_add = [&](int l, double Pb, double Pt, double tpd, float hq, float w, float dl, double sgn) {
@@ -467,7 +485,7 @@ pgw_column_tma_kernel(const __grid_constant__ pgw_timestep_args a, const __grid_
             const double2 hl = s_hl[l];
             const double Pt = fma(PSd, hl.y, hl.x);
             double pt = Pt;
-            if (pt < pref) { pt = pref; era_open = false; lstar = l; }   // layer that contains p_ref (:174-179)
+            if (pt < pref) { pt = pref; era_open = false; s_lstar[ct] = l; }   // layer that contains p_ref (:174-179)
             const double td = (double)t, tpd = (double)t_pgw;
             const double rtv = rd_tv(t, q);                          // Rd * Tv of the ERA state, float32 products
             const float g = fast_rcp(fmaf(-0.378f, e_pgw, p));
@@ -493,18 +511,29 @@ pgw_column_tma_kernel(const __grid_constant__ pgw_timestep_args a, const __grid_
         const double fis = (double)r_fis;
         const double phi_era = fis + acc_era;                            // acc_era holds Rd * Tv * dlnp
         const double gdzg = blend_f64(a.zg_ref, r_zg) * kG;              // step_03:292-295
-        const float2 *const bTe = st_Te + (size_t)(L - 1 - lst) * NT + tid;  // lowest level of the stash
         const double t_low = t_low_d;                                 // ta_pgw on the lowest level
+        int lstar = s_lstar[ct];
         const bool no_star = lstar < 0;                               // p_ref not reached among the parked levels
         if (no_star) lstar = lst;
         const double acc_k0 = acc_T0 + acc_part0;                     // iteration 0: x = 0, all layers
         // the layer right below l* joins the directly integrated ones: take it out of the polynomial
         const int ld_hi = min(lstar + 1, L - 1), ld_lo = max(lstar - 1, lst);
+        auto scol = [&](int l) { return tm + (uint32_t)(2 * (L - 1 - l)); };   // stash columns of level l
+        tmem_wait_st();
+        // (T_pgw, e_pgw) of the directly integrated layers ld_hi, ld_hi-1, ld_hi-2 (>= ld_lo) in registers.  The
+        // lanes' layers differ and a TMEM load takes one column address per warp: walk the warp's range.
+        float2 te_d0 = make_float2(0.f, 0.f), te_d1 = te_d0, te_d2 = te_d0;
+        for (int l = __reduce_max_sync(0xffffffffu, ld_hi), lo = __reduce_min_sync(0xffffffffu, ld_lo); l >= lo; --l) {
+            const float2 v = tmem_ld2(scol(l));
+            if (l == ld_hi) te_d0 = v;
+            if (l == ld_hi - 1) te_d1 = v;
+            if (l == ld_hi - 2) te_d2 = v;
+        }
         if (lstar + 1 <= L - 1) {
             const int l = lstar + 1;
             const double2 ht = s_hl[l], hb = s_hl[l + 1];
             const float2 m = s_m[l];
-            const float2 te = bTe[-(L - 1 - l) * NT];
+            const float2 te = te_d0;                                  // l == ld_hi
             const double Pt = fma(PSd, ht.y, ht.x), Pb = fma(PSd, hb.y, hb.x);
             const float g = fast_rcp(fmaf(-0.378f, te.y, fmaf(ps_f, m.y, m.x)));
             const float hq_t = (0.61f * 0.622f) * te.y * g;
@@ -547,12 +576,11 @@ pgw_column_tma_kernel(const __grid_constant__ pgw_timestep_args a, const __grid_
                 acc = fma(dps, fma(dps, fma(dps, fma(dps, c4, c3), c2), c1), acc + acc_T0);
                 // the layers around p_ref, top-down from the polynomial's upper edge (functions.py:174-179)
                 pb = p_edge;
-                const float2 *pTe = bTe - (L - 1 - ld_hi) * NT;
-                for (int l = ld_hi; l >= ld_lo; --l, pTe -= NT) {
+                for (int l = ld_hi; l >= ld_lo; --l) {
                     const double2 hl = s_hl[l];
                     const double pt = fma(psn, hl.y, hl.x);
                     const bool part = pt < pref;
-                    acc = layer(l, *pTe, part ? pref : pt, acc);
+                    acc = layer(l, l == ld_hi ? te_d0 : (l == ld_hi - 1 ? te_d1 : te_d2), part ? pref : pt, acc);
                     pb = pt;
                     if (part) break;
                 }
@@ -561,16 +589,25 @@ pgw_column_tma_kernel(const __grid_constant__ pgw_timestep_args a, const __grid_
                 // layers ltop..L-1 are entirely below p_ref for this ps; it moves by at most a level or two
                 while (ltop > lst) { const double2 h = s_hl[ltop - 1]; if (fma(psn, h.y, h.x) >= pref) --ltop; else break; }
                 while (ltop < L) { const double2 h = s_hl[ltop]; if (fma(psn, h.y, h.x) < pref) ++ltop; else break; }
-                const float2 *pTe = bTe;
-                int l = L - 1;
-#pragma unroll 2
-                for (; l >= ltop; --l, pTe -= NT) {
-                    const double2 hl = s_hl[l];
-                    const double pt = fma(psn, hl.y, hl.x);
-                    acc = layer(l, *pTe, pt, acc);
-                    pb = pt;
+                // bottom-up: the whole layers ltop..L-1, then ltop-1 (>= lst) up to p_ref if it lies below it
+                // (:174-179).  The stash is read for the whole warp, four levels per load, as far as any lane goes.
+                const int nlv = __reduce_max_sync(0xffffffffu, min(L - ltop + 1, np));
+#pragma unroll 1
+                for (int g = 0; g < nlv; g += 4) {
+                    float v[8];
+                    tmem_ld8(tm + (uint32_t)(2 * g), v);
+#pragma unroll
+                    for (int q = 0; q < 4; ++q) {
+                        const int l = L - 1 - g - q;
+                        const bool whole = l >= ltop, part = !whole && l == ltop - 1 && l >= lst && pb >= pref;
+                        if (whole || part) {
+                            const double2 hl = s_hl[l];
+                            const double pt = whole ? fma(psn, hl.y, hl.x) : pref;
+                            acc = layer(l, make_float2(v[2 * q], v[2 * q + 1]), pt, acc);
+                            pb = pt;
+                        }
+                    }
                 }
-                if (l >= lst && pb >= pref) acc = layer(l, *pTe, pref, acc);   // layer that contains p_ref (:174-179)
             }
             const double phi_pgw = fis + kRd * acc;
             const double err = (phi_pgw - phi_era) - gdzg;
@@ -585,24 +622,39 @@ pgw_column_tma_kernel(const __grid_constant__ pgw_timestep_args a, const __grid_
             a.PS_out[c] = psn_f;
             a.dps_out[c] = (float)dps;
         }
-        const float2 *pTe = bTe;
         uint32_t o2 = (uint32_t)(L - 1) * n + c;
         float *const oQ = a.QV_out;
-        for (int l = L - 1; l >= lst; --l, pTe -= NT, o2 -= n) {
-            const float qv = qv_from_e(pTe->y, psn_f, s_m[l]);
-            if (valid) st_stream(oQ + o2, qv);
+#pragma unroll 1
+        for (int g = 0; g < np; g += 8) {
+            float v[16];
+            tmem_ld16(tm + (uint32_t)(2 * g), v);          // levels L-1-g .. L-8-g
+#pragma unroll
+            for (int q = 0; q < 8; ++q) {
+                const int l = L - 1 - g - q;
+                if (l >= lst) {
+                    const float qv = qv_from_e(v[2 * q + 1], psn_f, s_m[l]);
+                    if (valid) st_stream(oQ + o2, qv);
+                    o2 -= n;
+                }
+            }
+        }
+        // the stash is dead: give the columns back now rather than at exit (the next CTA on this SM waits for them)
+        tmem_fence_before_sync();
+        asm volatile("bar.sync 1, %0;" ::"n"(NT) : "memory");    // the four column warps
+        if (ct < 32) {
+            tmem_fence_after_sync();
+            tmem_dealloc(tm, ncols);
         }
     };
 
     // ---------------- the sweep: parked pairs, fixed point, streamed pairs ----------------
-    float2 *pTe = st_Te + (size_t)(L - 1 - lst) * NT + tid;
     // one level pair; `parked` is a compile-time tag so that each of the two loops below gets its own body
     auto pair_body = [&](const int j, auto parked_c) {
         constexpr bool parked = decltype(parked_c)::value;
         const int l = max(L - 1 - 2 * j, 1);          // last pair of an odd column: levels (1, 0) again
         float2 mm0, mm1;
         if (parked) { mm0 = s_m[l]; mm1 = s_m[l - 1]; } else { mm0 = tp.m[l]; mm1 = tp.m[l - 1]; }
-        float *const sl = ring + (j % kTmaSlots) * 8 * NT + tid;
+        float *const sl = ring + (j % kTmaSlots) * 8 * NT + ct;
         // the walks need no slot data: they cover the round trip of the barrier probe (~100 cycles)
         const bool ready = mbar_test(bar_full + (j % kTmaSlots), (j / kTmaSlots) & 1);
 #if PGW_X2
@@ -648,9 +700,7 @@ pgw_column_tma_kernel(const __grid_constant__ pgw_timestep_args a, const __grid_
         if (parked) {
             fence_proxy_async();
             mbar_arrive(bar_done + (j % kTmaSlots));
-            pTe[0] = make_float2(tp0, e0);
-            pTe[-NT] = make_float2(tp1, e1);
-            pTe -= 2 * NT;
+            tmem_st4(tm + (uint32_t)(4 * j), tp0, e0, tp1, e1);     // levels l, l-1 = L-1-2j, L-2-2j
             if (j == 0) t_low_d = (double)t0 + (double)d0.ta;
             era_layer(l, p0, mm0.y, t0, q0, d0.ta, tp0, e0);
             era_layer(l - 1, p1, mm1.y, t1, q1, d1.ta, tp1, e1);
@@ -712,17 +762,31 @@ namespace {
 
 using pgw::kColumnThreads;
 
+// sm_100: 228 KB of shared memory and 512 tensor-memory columns per SM, 1 KB of shared memory reserved per CTA
+constexpr size_t kSmemPerSm = 228 * 1024, kSmemReservedPerCta = 1024;
+constexpr int kTmemColsPerSm = 512;
+
+// tensor-memory columns of a CTA: (T_pgw, e_pgw) of np levels, allocated in powers of two >= 32
+int tmem_cols_tma(int np) {
+    int c = 32;
+    while (c < 2 * np) c <<= 1;
+    return c;
+}
+
+// Shared memory per CTA.  It is padded to the CTA's share of the SM's tensor memory, so that the CTAs that fit by
+// shared memory (of this kernel, whichever plan, e.g. the next launch on another stream) also fit by tensor memory
+// and tcgen05.alloc never waits: 128 columns -> 56 KB (4 CTAs, the register limit anyway), 256 -> 113 KB, 512 -> 227 KB.
 size_t column_smem_tma(int nplev, int np, int nlev) {
     const int nt = kColumnThreads;
     size_t b = sizeof(float) * (size_t)pgw::kTmaSlots * 8 * nt +            // pair ring
-               (size_t)np * nt * (2 * sizeof(float)) +                      // stash
                sizeof(double) * 2 * (size_t)(np + 1) + sizeof(float) * 2 * (size_t)np;
     b += sizeof(float) * (size_t)(3 * nplev + ((3 * nplev) & 1));
 #if PGW_UNIFORM_TOP
     b += 2 * sizeof(float) * (size_t)(nlev + (nlev & 1));
 #endif
-    b += sizeof(uint64_t) * 2 * pgw::kTmaSlots;
-    return b;
+    b += sizeof(uint64_t) * 2 * pgw::kTmaSlots + sizeof(uint32_t) * (1 + nt);   // barriers, TMEM address, l*
+    const size_t share = kSmemPerSm * (size_t)tmem_cols_tma(np) / kTmemColsPerSm - kSmemReservedPerCta;
+    return b > share ? b : share;
 }
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
@@ -815,6 +879,15 @@ int pgw_launch_column_tma(const pgw_timestep_args *a, const pgw_column_plan &pla
     if ((rc = pgw_ensure_smem((const void *)kern, 4 + (plan.fast ? 1 : 0) + (l137 ? 2 : 0), plan.smem, plan.np)) != PGW_OK)
         return rc;
     const unsigned grid = (unsigned)((a->ncol + kColumnThreads - 1) / kColumnThreads);
-    kern<<<grid, kColumnThreads + 32, plan.smem, st>>>(*a, tp, plan.lst, plan.np);
+    kern<<<grid, 2 * kColumnThreads, plan.smem, st>>>(*a, tp, plan.lst, plan.np, (uint32_t)tmem_cols_tma(plan.np));
     return pgw_check_launch("pgw_column_tma_kernel");
+}
+
+extern "C" int pgw_column_tma_layout(int nplev, int nlev, int np, int *tmem_cols, long long *smem_bytes) {
+    if (nplev < 2 || nplev > 64 || nlev < 2 || nlev > pgw::kTmaMaxLev || np < 2 || np > nlev || (np & 1) ||
+        !tmem_cols || !smem_bytes)
+        return PGW_E_INVALID;
+    *tmem_cols = tmem_cols_tma(np);
+    *smem_bytes = (long long)column_smem_tma(nplev, np, nlev);
+    return PGW_OK;
 }
