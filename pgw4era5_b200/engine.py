@@ -47,6 +47,16 @@ def _stream():
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
+def fused_refusal():
+    """Why ``PGWEngine.submit`` cannot run the current settings in the fused pass (None if it can)."""
+    ref_dtypes = getattr(settings, "i_reference_dtypes", 0)
+    if (settings.i_reinterp and settings.p_ref_inp is None) or \
+            ((settings.i_reinterp or settings.p_ref_inp is None) and ref_dtypes):
+        return ("i_reinterp = 1 with p_ref_inp = None, and either of them with i_reference_dtypes = 1, "
+                "run through the staged path: use apply()")
+    return None
+
+
 def read_axes(name, d):
     """(kept stamps, indices of the kept stamps in the source, plev or None) of one delta variable in the dict
     form ``DeltaSet`` takes; 29 February is dropped (functions.py:224-230)."""
@@ -350,11 +360,9 @@ class PGWEngine:
         T, QV, U, V [1,L,ny,nx] (the names of settings.var_name_map).  Returns a
         ``Pending``; nothing is synchronised here.
         """
-        ref_dtypes = getattr(settings, "i_reference_dtypes", 0)
-        if (settings.i_reinterp and settings.p_ref_inp is None) or \
-                ((settings.i_reinterp or settings.p_ref_inp is None) and ref_dtypes):
-            raise ValueError("i_reinterp = 1 with p_ref_inp = None, and either of them with i_reference_dtypes = 1, "
-                             "run through the staged path: use apply()")
+        msg = fused_refusal()
+        if msg is not None:
+            raise ValueError(msg)
         a, f, out, ws, k_spec, k_max = self._fill_args(era, era_step_dt, out, k_spec, slot)
         if direct:
             a.flags |= N.FLAG_DIRECT          # every parked level integrated in every iteration

@@ -6,9 +6,9 @@ intermediate numpy copies.  NetCDF-3 stores big-endian numbers; the byte order o
 fields is swapped on the GPU (``pgw_byteswap32``), next to the H2D / D2H copies.
 
 Only what the pipeline needs: locate a variable (offset, shape, type) and read or overwrite the
-values of one record.  Everything else (coordinates, attributes, the engine's level tables) goes
-through ``ncio``.  File format: NetCDF Classic Format Specification (Unidata), all integers
-big-endian:
+values of one record, or of a band of its rows (latitude-band mode).  Everything else (coordinates,
+attributes, the engine's level tables) goes through ``ncio``.  File format: NetCDF Classic Format
+Specification (Unidata), all integers big-endian:
     header  = magic numrecs dim_list gatt_list var_list
     var     = name nelems [dimid ...] vatt_list nc_type vsize begin
 """
@@ -226,3 +226,51 @@ class RawNC3:
         off, done = self.offset(name, record), 0
         while done < mv.nbytes:
             done += os.pwrite(fd, mv[done:], off + done)
+
+    def _row_pieces(self, name, nbytes, r0, r1, record):
+        """(file offset, buffer offset, bytes) of every contiguous piece of rows [r0, r1) of the second-to-last
+        axis of ``name``, for every index of the axes in front of it; the buffer holds the band as
+        [..., r1 - r0, nx]."""
+        v = self.vars[name]
+        shp = v.record_shape
+        if len(shp) < 2:
+            raise ValueError("%s has no row axis" % name)
+        ny, row = shp[-2], shp[-1] * v.dtype.itemsize
+        lead = int(np.prod(shp[:-2], dtype=np.int64))
+        if not 0 <= r0 < r1 <= ny:
+            raise ValueError("%s: rows %d..%d of %d" % (name, r0, r1, ny))
+        if not v.is_record and record != 0:
+            raise IndexError("%s is not a record variable" % name)
+        band = (r1 - r0) * row
+        if nbytes != lead * band:
+            raise ValueError("%s: buffer has %d bytes, rows %d..%d %d" % (name, nbytes, r0, r1, lead * band))
+        base = self.offset(name, record)
+        if r1 - r0 == ny:                            # whole rows of every level: one piece
+            return [(base, 0, lead * band)]
+        return [(base + (i * ny + r0) * row, i * band, band) for i in range(lead)]
+
+    def read_rows(self, fobj, name, buf, r0, r1, record=0):
+        """Fill ``buf`` with the raw big-endian bytes of rows [r0, r1) of ``name`` (the second-to-last axis; every
+        index of the axes in front of it, e.g. levels), stored contiguously as [..., r1 - r0, nx]."""
+        pieces = self._row_pieces(name, memoryview(buf).nbytes, r0, r1, record)
+        mv = memoryview(buf).cast("B")
+        for off, pos, count in pieces:
+            done = 0
+            while done < count:
+                n = os.preadv(fobj.fileno(), [mv[pos + done:pos + count]], off + done)
+                if n <= 0:
+                    raise IOError("unexpected end of %s while reading %s" % (self.path, name))
+                done += n
+
+    def write_rows(self, fd, name, buf, r0, r1, record=0):
+        """Overwrite rows [r0, r1) of ``name`` in the file open as descriptor ``fd`` with the raw big-endian bytes
+        of ``buf`` (laid out as ``read_rows`` fills it); the other rows are left as they are."""
+        pieces = self._row_pieces(name, memoryview(buf).nbytes, r0, r1, record)
+        mv = memoryview(buf).cast("B")
+        for off, pos, count in pieces:
+            done = 0
+            while done < count:
+                n = os.pwrite(fd, mv[pos + done:pos + count], off + done)
+                if n <= 0:
+                    raise IOError("short write of %s to %s" % (name, self.path))
+                done += n

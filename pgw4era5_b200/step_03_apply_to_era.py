@@ -7,6 +7,11 @@ Same command line (``-i -o -f -l -H -d -p -t -D``), same ``settings.py`` names, 
 naming; the per-file work (step_03_apply_to_era.py:44-381 of the reference) runs as one fused
 CUDA pass per ERA5 file on a B200 through ``PGWEngine``.  ``-p N`` starts N worker processes,
 worker i bound to GPU i % device_count (the reference's pool of CPU workers, parallel.py).
+``--latitude_bands`` (under torchrun, not in the reference) splits every file into latitude bands instead, one
+rank per GPU, each rank reading, computing and writing its own rows (``pgw_for_era5_files(band=...)``):
+
+    torchrun --standalone --nproc-per-node 8 -m pgw4era5_b200.step_03_apply_to_era \\
+           -i era_in -o era_out -d deltas -f 2006080200 -l 2006080200 -H 3 -t --latitude_bands
 
     python -m pgw4era5_b200.step_03_apply_to_era -i era_in -o era_out -d deltas \\
            -f 2006080200 -l 2006080300 -H 3 -t
@@ -14,6 +19,7 @@ worker i bound to GPU i % device_count (the reference's pool of CPU workers, par
 import argparse
 import os
 from argparse import RawDescriptionHelpFormatter
+from collections import namedtuple
 from datetime import datetime, timedelta
 from pathlib import Path
 
@@ -25,43 +31,110 @@ from .parallel import IterMP
 _ENGINES = {}
 
 
-def load_delta_set(delta_input_dir, device="cuda", max_resident_bytes=None):
+def load_delta_set(delta_input_dir, device="cuda", max_resident_bytes=None, rows=None):
     """Read every delta file the path needs (ta, hur, ua, va, zg, tas, hurs, ts, tos, siconc as
     SCEN-HIST, ps as HIST; step_03_apply_to_era.py:533-539) into one device-resident DeltaSet, or, when
     that set and the staging copy of one variable would take more than ``max_resident_bytes`` (default:
     half of the device's free memory), into a ``StreamedDeltaSet`` that reads the 3-D deltas of NetCDF-3
-    files stamp by stamp.  Only the headers and coordinates of the 3-D files are read to decide."""
+    files stamp by stamp.  Only the headers and coordinates of the 3-D files are read to decide.
+
+    ``rows = (r0, r1)``: a resident DeltaSet of those latitude rows only (latitude-band mode); the 3-D deltas of
+    NetCDF-3 files are read band by band with ``RawNC3.read_rows``, other files are decoded and sliced.  A band
+    set is never streamed: one that exceeds the limit raises ValueError before anything is uploaded."""
     from . import deltastream
     from .engine import DeltaSet, VARS_2D, VARS_3D
     headers = deltastream.read_3d_headers(delta_input_dir)
-    if deltastream.should_stream(headers, device, max_resident_bytes):
+    if rows is not None and headers is not None:
+        ta = headers["ta"][0].vars[headers["ta"][1]]
+        _check_band_fits(deltastream.resident_bytes(headers), ta.shape[-2], device, max_resident_bytes, rows)
+    elif rows is None and deltastream.should_stream(headers, device, max_resident_bytes):
         return deltastream.open_streamed(delta_input_dir, headers, device=device)
-    deltas = {}
+    deltas, decoded_bytes = {}, []
     for name in VARS_3D + VARS_2D:
+        if rows is not None and headers is not None and name in VARS_3D:
+            raw, var_name, axes = headers[name]
+            deltas[name] = dict(axes, data=_read_band(raw, var_name, rows))
+            continue
         path, var_name = deltastream.delta_file(delta_input_dir, name)
         ds = ncio.open_dataset(path)
         var = ds[var_name]
         plev = None
         if settings.PLEV_GCM in var.dims:
             plev = np.asarray(ds[settings.PLEV_GCM].data, dtype=np.float64)
-        deltas[name] = dict(time=ncio.decode_time(ds[settings.TIME_GCM]), plev=plev, data=var.data)
+        decoded_bytes.append(4 * int(var.data.size))
+        ny = var.data.shape[-2]
+        data = var.data if rows is None else np.ascontiguousarray(var.data[..., rows[0]:rows[1], :])
+        deltas[name] = dict(time=ncio.decode_time(ds[settings.TIME_GCM]), plev=plev, data=data)
+    if rows is not None and headers is None:
+        # decoded 3-D deltas: the whole set as DeltaSet would hold it (its arena, plus the staging copy of the
+        # largest variable), sized from the decoded arrays; 29 February counted, so an upper bound
+        _check_band_fits(sum(decoded_bytes) + max(decoded_bytes), ny, device, max_resident_bytes, rows)
     return DeltaSet(deltas, device=device)
 
 
-def get_engine(delta_input_dir, era_file):
-    """One engine (and one resident copy of the climatology) per process and delta directory."""
+def _read_band(raw, name, rows):
+    """Rows [r0, r1) of a 4-D float32 variable of a NetCDF-3 file as a native-endian array, entry by entry of its
+    first axis (record by record for a record variable)."""
+    v = raw.vars[name]
+    r0, r1 = rows
+    out = np.empty(v.shape[:-2] + (r1 - r0, v.shape[-1]), dtype=v.dtype)
+    with open(raw.path, "rb", buffering=0) as f:
+        if v.is_record:
+            for rec in range(raw.numrecs):
+                raw.read_rows(f, name, out[rec], r0, r1, record=rec)
+        else:
+            raw.read_rows(f, name, out, r0, r1)
+    return out.byteswap(inplace=True).view(v.dtype.newbyteorder("="))
+
+
+def _check_band_fits(whole, ny, device, max_resident_bytes, rows):
+    """ValueError when the band of a delta set that needs ``whole`` bytes of device memory for all ``ny`` rows
+    (linear in the number of rows) needs more than ``max_resident_bytes`` (default: half of the device's free
+    memory), naming the number of ranks whose bands would fit."""
+    import torch
+    from .parallel import split_rows
+    if max_resident_bytes is None:
+        max_resident_bytes = torch.cuda.mem_get_info(torch.device(device))[0] // 2
+    need = whole * (rows[1] - rows[0]) // ny
+    if need <= max_resident_bytes:
+        return
+    fit = next((w for w in range(1, ny + 1) if whole * max(b - a for a, b in split_rows(ny, w)) // ny
+                <= max_resident_bytes), None)
+    raise ValueError("the delta band of rows %d..%d needs %.2f GB on the device, more than the %.2f GB allowed; "
+                     "a latitude-band set is always resident: %s" % (
+                         rows[0], rows[1], need / 1e9, max_resident_bytes / 1e9,
+                         "%d ranks or more would fit" % fit if fit else "no number of ranks fits"))
+
+
+def get_engine(delta_input_dir, era_file, band=None):
+    """One engine (and one resident copy of the climatology) per process and delta directory; with ``band``
+    (latitude-band mode, ``Band``) one per row range, holding the deltas of those rows only."""
     import torch
     from .engine import PGWEngine
     ak = np.asarray(era_file['ak'].data)
     bk = np.asarray(era_file['bk'].data)
     key = (os.path.abspath(delta_input_dir), torch.cuda.current_device(), ak.tobytes(), bk.tobytes())
+    if band is not None:
+        key += (tuple(band.rows), band.exchange)
     eng = _ENGINES.get(key)
     if eng is None:
-        ds = load_delta_set(delta_input_dir, device=torch.device("cuda", torch.cuda.current_device()))
+        device = torch.device("cuda", torch.cuda.current_device())
+        if band is None:
+            ds = load_delta_set(delta_input_dir, device=device)
+        else:
+            # a band that does not fit, or a delta file one rank cannot read, must stop every rank before the
+            # engine's first collective
+            ds, err = None, None
+            try:
+                ds = load_delta_set(delta_input_dir, device=device, rows=band.rows)
+            except Exception as e:
+                err = e
+            _agree_or_raise(band, err, 0, "loading the delta climatology")
         akm = np.asarray(era_file['akm'].data) if 'akm' in era_file else None      # step_03:68-85
         bkm = np.asarray(era_file['bkm'].data) if 'bkm' in era_file else None
         soil = np.asarray(era_file[settings.SOIL_HLEV_ERA].data) if settings.SOIL_HLEV_ERA in era_file else ()
-        eng = PGWEngine(ak, bk, ds, soil1=soil, akm=akm, bkm=bkm)
+        eng = PGWEngine(ak, bk, ds, soil1=soil, akm=akm, bkm=bkm,
+                        **({} if band is None else dict(group=band.group, band_exchange=band.exchange)))
         _ENGINES[key] = eng
     return eng
 
@@ -141,10 +214,12 @@ def _out_dtype(key, file_dtype):
 IO_STATS = {"raw": 0, "decoded": 0}          # files per I/O path of pgw_for_era5_files (tests, bench_files.py)
 
 
-def _raw_layout(path, names, host_in):
+def _raw_layout(path, names, host_in, grid=None):
     """The header of ``path`` if the file can go through the pipeline without decoding: NetCDF-3, one
     record at most, every ERA5 field float32 with the size of its host buffer, no RELHUM to drop
-    (step_03:371).  Else None (the decoding path is taken)."""
+    (step_03:371).  Else None (the decoding path is taken).  ``grid = (ny, nx)``: the host buffers hold a
+    band of rows of that grid (latitude-band mode), so the fields must have ``grid`` as their last two axes
+    and the buffers as many rows of every level as the band has."""
     from .nc3raw import NC_FLOAT, NotNetCDF3, RawNC3
     if os.environ.get("PGW_RAW_IO", "1") == "0" or getattr(settings, "i_reference_output_dtypes", 0):
         return None                 # float64 outputs change the layout of the file: decoding path
@@ -156,8 +231,14 @@ def _raw_layout(path, names, host_in):
         return None
     for key, name in names.items():
         v = raw.vars.get(name)
-        if v is None or v.nc_type != NC_FLOAT or (v.is_record and raw.numrecs != 1) or \
-                v.nbytes != host_in[key].numel() * 4:
+        if v is None or v.nc_type != NC_FLOAT or (v.is_record and raw.numrecs != 1):
+            return None
+        if grid is None:
+            if v.nbytes != host_in[key].numel() * 4:
+                return None
+        elif tuple(v.record_shape[-2:]) != tuple(grid) or \
+                v.nbytes // (grid[0] * grid[1]) * host_in[key].shape[-2] * grid[1] != host_in[key].numel() * 4 or \
+                host_in[key].shape[-1] != grid[1]:
             return None
     return raw
 
@@ -181,7 +262,9 @@ _WRITE_PIECE = 64 << 20
 def _write_raw(raw, names, inp_path, out_path, host_out, pool=None):
     """The output file = the input file with the eight updated fields replaced (step_03:367-378): the
     bytes in between are copied file to file, the fields come straight from the (big-endian) host buffers.
-    All writes are positional, so ``pool`` (a ThreadPoolExecutor) may run them side by side."""
+    All writes are positional, so ``pool`` (a ThreadPoolExecutor) may run them side by side.  ``host_out = None``:
+    the file gets the input's size and every byte outside the eight fields, whose rows the ranks of a
+    latitude-band run then write (``RawNC3.write_rows``)."""
     segs = sorted((raw.offset(names[k]), raw.vars[names[k]].nbytes, k) for k in _WRITTEN)
     fd_in = os.open(inp_path, os.O_RDONLY)
     fd_out = os.open(out_path, os.O_WRONLY | os.O_CREAT | os.O_TRUNC, 0o644)
@@ -198,9 +281,10 @@ def _write_raw(raw, names, inp_path, out_path, host_out, pool=None):
         jobs, pos = [], 0
         for off, nbytes, key in segs:
             jobs.append((_copy_range, (fd_in, fd_out, pos, off - pos)))
-            # a 3-D field of a global file is 570 MB: cut into pieces so that all writer threads stay busy
-            for lo in range(0, nbytes, _WRITE_PIECE):
-                jobs.append((put, (off, nbytes, key, lo, min(nbytes, lo + _WRITE_PIECE))))
+            if host_out is not None:
+                # a 3-D field of a global file is 570 MB: cut into pieces so that all writer threads stay busy
+                for lo in range(0, nbytes, _WRITE_PIECE):
+                    jobs.append((put, (off, nbytes, key, lo, min(nbytes, lo + _WRITE_PIECE))))
             pos = off + nbytes
         jobs.append((_copy_range, (fd_in, fd_out, pos, size - pos)))
         if pool is None:
@@ -214,7 +298,138 @@ def _write_raw(raw, names, inp_path, out_path, host_out, pool=None):
         os.close(fd_out)
 
 
-def pgw_for_era5_files(steps, delta_input_dir, ignore_top_pressure_error, debug_mode=None):
+def _write_band(raw, names, out_path, host_out, rows, pool=None):
+    """Rows [r0, r1) of the eight written fields from the (big-endian) band buffers ``host_out`` into the output
+    file that rank 0 prepared (``_write_raw`` without buffers)."""
+    fd = os.open(out_path, os.O_WRONLY)
+    try:
+        jobs = [(raw.write_rows, (fd, names[k], host_out[k].numpy(), rows[0], rows[1])) for k in _WRITTEN]
+        if pool is None:
+            for fn, args in jobs:
+                fn(*args)
+        else:
+            for fut in [pool.submit(fn, *args) for fn, args in jobs]:
+                fut.result()
+    finally:
+        os.close(fd)
+
+
+class Band(namedtuple("Band", "group host_group rows exchange")):
+    """This rank's share of a latitude-band run: ``group`` the (NCCL) process group the engine merges its status
+    block over, ``host_group`` a gloo group of the same ranks for the host-side agreement (it waits on no CUDA
+    stream), ``rows = (r0, r1)`` the latitude rows of this rank (None: ``split_rows(ny, world)[rank]`` of the
+    files' grid), ``exchange`` the engine's ``band_exchange``."""
+    __slots__ = ()
+
+    def __new__(cls, group, host_group, rows=None, exchange="auto"):
+        return super().__new__(cls, group, host_group, None if rows is None else tuple(rows), exchange)
+
+
+def _agree_or_raise(band, err, fingerprint, what):
+    """Every rank of ``band`` learns whether any rank failed (``err``) at this point, and whether all of them saw
+    the same ``fingerprint``: one all-reduce (MAX) on the gloo group.  A failure raises on every rank -- its own
+    exception on the rank that failed, RuntimeError on the others -- so that no rank is left waiting in a
+    collective its peers never reach."""
+    import torch
+    import torch.distributed as dist
+    world, rank = dist.get_world_size(band.host_group), dist.get_rank(band.host_group)
+    v = torch.zeros(world + 2, dtype=torch.int64)
+    v[rank] = int(err is not None)
+    v[world], v[world + 1] = int(fingerprint), -int(fingerprint)
+    dist.all_reduce(v, op=dist.ReduceOp.MAX, group=band.host_group)
+    failed = [r for r in range(world) if int(v[r])]
+    if err is not None:
+        raise err
+    if failed:
+        raise RuntimeError("latitude bands: rank(s) %s failed while %s" % (failed, what))
+    if int(v[world]) != -int(v[world + 1]):
+        raise ValueError("latitude bands: the ranks disagree while %s (different files or headers)" % what)
+
+
+def _fingerprint(*parts):
+    """A 31-bit digest of ``parts`` (their repr) for ``_agree_or_raise``."""
+    import zlib
+    return zlib.crc32(repr(parts).encode()) & 0x7FFFFFFF
+
+
+def _layout_key(raw, names):
+    return tuple((names[k], raw.offset(names[k]), raw.vars[names[k]].shape) for k in sorted(names))
+
+
+MSG_BAND_FILES = ("latitude bands read and write ERA5 files in place: they need NetCDF-3 files with one record, "
+                  "float32 fields of one grid and no {} variable, and an output path other than the input")
+
+
+def _band_refusal(debug_mode):
+    """Why band mode cannot run the current settings (None if it can)."""
+    from .engine import fused_refusal
+    if debug_mode is not None:
+        return "latitude bands do not run the debug modes (-D)"
+    if getattr(settings, "i_reference_output_dtypes", 0):
+        return "latitude bands write the input file's layout: i_reference_output_dtypes = 1 is not supported"
+    if os.environ.get("PGW_RAW_IO", "1") == "0":
+        return "latitude bands need the raw NetCDF-3 path (PGW_RAW_IO=0 is set)"
+    return fused_refusal()
+
+
+def _level_tables(path, names):
+    """What the engine needs from the first ERA5 file -- ak, bk (akm, bkm and the soil depths where present) --
+    as an ``ncio.Dataset`` read from the NetCDF-3 header and those small variables, and the grid (ny, nx) from
+    the header of PS.  No field is read."""
+    from .nc3raw import NotNetCDF3, RawNC3
+    try:
+        raw = RawNC3(path)
+    except (NotNetCDF3, OSError) as e:
+        raise ValueError("%s: %s (%s)" % (path, MSG_BAND_FILES.format(settings.var_name_map['hur']), e))
+    if names["PS"] not in raw.vars or "ak" not in raw.vars or "bk" not in raw.vars:
+        raise ValueError("%s: %s" % (path, MSG_BAND_FILES.format(settings.var_name_map['hur'])))
+    out = ncio.Dataset()
+    with open(path, "rb", buffering=0) as f:
+        for name in ("ak", "bk", "akm", "bkm", settings.SOIL_HLEV_ERA):
+            if name in raw.vars:
+                v = raw.vars[name]
+                out[name] = ncio.Variable(v.dims, raw.read_variable(f, name), v.attrs)
+    ny, nx = raw.vars[names["PS"]].record_shape[-2:]
+    return out, (int(ny), int(nx))
+
+
+def _band_start(steps, names, band):
+    """Latitude-band mode before any GPU work: the grid and this rank's rows from the first file, every input
+    file checked on every rank, the output files created by rank 0 (the input's bytes outside the eight written
+    fields), then the start barrier -- an agreement on the gloo group.  Every rank reads headers and level tables
+    only, never a whole field.  Returns (level tables of the first file, (ny, nx), rows)."""
+    import torch
+    import torch.distributed as dist
+    from .parallel import split_rows
+    vmap = settings.var_name_map
+    err, fp, first, grid, rows = None, 0, None, None, band.rows
+    try:
+        first, grid = _level_tables(steps[0]["inp_era_file_path"], names)
+        nx = grid[1]
+        if rows is None:
+            rows = split_rows(grid[0], dist.get_world_size(band.group))[dist.get_rank(band.group)]
+        nlev = len(first["ak"].data) - 1
+        nsoil = len(first[settings.SOIL_HLEV_ERA].data) if settings.SOIL_HLEV_ERA in first else 0
+        lev = dict(T_SO=nsoil, T=nlev, QV=nlev, U=nlev, V=nlev)
+        shapes = {k: torch.empty((1, lev.get(k, 1), rows[1] - rows[0], nx), device="meta") for k in names}
+        layouts = []
+        for st in steps:
+            inp, out = st["inp_era_file_path"], st["out_era_file_path"]
+            raw = _raw_layout(inp, names, shapes, grid=grid)
+            if raw is None or os.path.realpath(inp) == os.path.realpath(out):
+                raise ValueError("%s: %s" % (inp, MSG_BAND_FILES.format(vmap['hur'])))
+            layouts.append(_layout_key(raw, names))
+            if dist.get_rank(band.host_group) == 0:
+                _write_raw(raw, names, inp, out, None)
+        fp = _fingerprint(grid, [(st["inp_era_file_path"], st["out_era_file_path"], str(st["era_step_dt"]))
+                                 for st in steps], layouts)
+    except Exception as e:
+        err = e
+    _agree_or_raise(band, err, fp, "checking the input files and creating the output files")
+    return first, grid, tuple(rows)
+
+
+def pgw_for_era5_files(steps, delta_input_dir, ignore_top_pressure_error, debug_mode=None, band=None):
     """
     The production mode of ``pgw_for_era5`` for a LIST of files on one GPU, as a three-stage
     pipeline (SURVEY.md 8f rank 1): a reader thread decodes file i+1 into pinned host buffers and
@@ -225,6 +440,14 @@ def pgw_for_era5_files(steps, delta_input_dir, ignore_top_pressure_error, debug_
     the writer assembles the output from the input file and the result buffers.  Results are
     identical to calling ``pgw_for_era5`` file by file.  ``steps``: dicts with inp_era_file_path,
     out_era_file_path, era_step_dt.  Returns the iteration counts.
+
+    ``band`` (a ``Band``): latitude-band mode, every rank of ``band.group`` runs this with the same ``steps``.
+    Rank 0 creates the output files first; each rank then reads its rows of every field (``RawNC3.read_rows``),
+    runs them through an engine over its rows of the deltas whose status block is merged over the ranks, and
+    writes its rows into the shared output files (``RawNC3.write_rows``).  The ranks agree on the gloo group
+    before the start, before each file's submit and at the end, so a failure on one rank raises on all of them.
+    Band mode runs whatever ``PGWEngine.submit`` runs (not the staged path, whose convergence test is per rank)
+    on NetCDF-3 files; other settings and files raise ValueError before any GPU work.
     """
     import queue
     import threading
@@ -232,16 +455,25 @@ def pgw_for_era5_files(steps, delta_input_dir, ignore_top_pressure_error, debug_
     from .hostpipe import HostPipeline, IN_FIELDS
     if not steps:
         return []
-    if debug_mode is not None or settings.i_reinterp or settings.p_ref_inp is None:
+    if band is not None:
+        msg = _band_refusal(debug_mode)
+        if msg is not None:
+            raise ValueError(msg)
+    elif debug_mode is not None or settings.i_reinterp or settings.p_ref_inp is None:
         return [pgw_for_era5(delta_input_dir=delta_input_dir,
                              ignore_top_pressure_error=ignore_top_pressure_error, debug_mode=debug_mode, **st)
                 for st in steps]
     vmap = settings.var_name_map
     names = _ERA_NAMES(vmap)
-    first = ncio.open_dataset(steps[0]["inp_era_file_path"], decode_cf=False)
-    eng = get_engine(delta_input_dir, first)
-    ny, nx = first[names["PS"]].data.shape[-2:]
-    pipe = HostPipeline(eng, ny, nx)
+    if band is None:
+        first = ncio.open_dataset(steps[0]["inp_era_file_path"], decode_cf=False)
+        ny, nx = first[names["PS"]].data.shape[-2:]
+        rows = (0, ny)
+    else:
+        first, (ny, nx), rows = _band_start(steps, names, band)
+        band = band._replace(rows=rows)
+    eng = get_engine(delta_input_dir, first, band)
+    pipe = HostPipeline(eng, rows[1] - rows[0], nx)
     n_in_buf, n_out_buf = 3, 4
     free_in, free_out = queue.Queue(), queue.Queue()
     for _ in range(n_in_buf):
@@ -282,11 +514,14 @@ def pgw_for_era5_files(steps, delta_input_dir, ignore_top_pressure_error, debug_
                 h = q_get(free_in)
                 if h is None:
                     return
-                raw = _raw_layout(st["inp_era_file_path"], names, h)
+                raw = _raw_layout(st["inp_era_file_path"], names, h, grid=None if band is None else (ny, nx))
+                if band is not None and raw is None:
+                    raise ValueError("%s: %s" % (st["inp_era_file_path"], MSG_BAND_FILES.format(vmap['hur'])))
                 if raw is not None and os.path.realpath(st["inp_era_file_path"]) != \
                         os.path.realpath(st["out_era_file_path"]):
+                    read = raw.read_into if band is None else (lambda f, n, b: raw.read_rows(f, n, b, *rows))
                     with open(st["inp_era_file_path"], "rb", buffering=0) as f:
-                        for fut in [rpool.submit(raw.read_into, f, names[key], h[key].numpy()) for key in IN_FIELDS]:
+                        for fut in [rpool.submit(read, f, names[key], h[key].numpy()) for key in IN_FIELDS]:
                             fut.result()
                     IO_STATS["raw"] += 1
                     if not q_put(loaded, (st, raw, h)):
@@ -311,6 +546,12 @@ def pgw_for_era5_files(steps, delta_input_dir, ignore_top_pressure_error, debug_
                 if item is None:
                     return
                 st, era_file, host = item
+                if band is not None:                                  # this rank's rows of the prepared file
+                    _write_band(era_file, names, st["out_era_file_path"], host, rows, wpool)
+                    free_out.put(host)
+                    if settings.i_debug >= 1:
+                        print('Done. Saved rows {}..{} to file {}.'.format(rows[0], rows[1], st["out_era_file_path"]))
+                    continue
                 if not isinstance(era_file, ncio.Dataset):           # raw layout
                     _write_raw(era_file, names, st["inp_era_file_path"], st["out_era_file_path"], host, wpool)
                     free_out.put(host)
@@ -346,20 +587,27 @@ def pgw_for_era5_files(steps, delta_input_dir, ignore_top_pressure_error, debug_
         to_write.put((st, era_file, h_out))
 
     try:
-        while True:
+        for k in range(len(steps)):
             item = q_get(loaded)
-            if item is None:
+            h_out = q_get(free_out) if item is not None else None
+            if band is not None:
+                # every rank read its band of file k (or none submits it): no column kernel or band exchange is
+                # launched that a peer would wait for in vain
+                ok = item is not None and h_out is not None and not failure
+                err = None if ok else (failure[0] if failure else RuntimeError("the file pipeline stopped"))
+                _agree_or_raise(band, err, _fingerprint(k, _layout_key(item[1], names)) if ok else 0,
+                                "reading %s" % steps[k]["inp_era_file_path"])
+            if item is None or h_out is None:
                 break
             st, era_file, h_in = item
-            h_out = q_get(free_out)
-            if h_out is None:
-                break
             done = pipe.run(h_in, st["era_step_dt"], h_out, raw=not isinstance(era_file, ncio.Dataset),
                             ignore_top_pressure_error=ignore_top_pressure_error, file_name=st["inp_era_file_path"])
             in_flight.append((st, era_file, h_in, h_out))
             if done is not None:
                 retire(done)
-        if not stop.is_set():
+        # band mode: every rank got here with every file submitted (the agreements above), and a rerun while
+        # draining is an exchange all ranks take part in, so a rank whose writer failed drains too
+        if band is not None or not stop.is_set():
             for done in pipe.drain():
                 if done is not None:
                     retire(done)
@@ -373,6 +621,8 @@ def pgw_for_era5_files(steps, delta_input_dir, ignore_top_pressure_error, debug_
         tr.join(timeout=5)
         rpool.shutdown(wait=False)
         wpool.shutdown(wait=False)
+    if band is not None:            # every output file is complete on every rank before any rank returns
+        _agree_or_raise(band, failure[0] if failure else None, len(n_iters), "writing the output files")
     if failure:
         raise failure[0]
     return n_iters
@@ -433,7 +683,40 @@ def build_parser():
     parser.add_argument('-D', '--debug_mode', type=str, default=None,
                         help='"interpolate_time": store the deltas interpolated in time only; '
                              '"interpolate_full": store the final deltas instead of the modified files.')
+    parser.add_argument('--latitude_bands', action='store_true',
+                        help='Run under torchrun, one rank per GPU: every rank reads, computes and writes its own '
+                             'latitude rows of each file, holding only those rows of the climate deltas '
+                             '(NetCDF-3 ERA5 files; not in the reference).')
     return parser
+
+
+def _check_band_args(args):
+    if args.n_par != 1:
+        raise ValueError('--latitude_bands runs one rank per GPU under torchrun: -p must be 1.')
+    if args.debug_mode is not None:
+        raise ValueError('--latitude_bands does not run the debug modes (-D).')
+    missing = [k for k in ("RANK", "WORLD_SIZE", "LOCAL_RANK") if k not in os.environ]
+    if missing:
+        raise ValueError('--latitude_bands needs the environment of torchrun (%s not set): start it as '
+                         'torchrun --nproc-per-node N -m pgw4era5_b200.step_03_apply_to_era ... --latitude_bands'
+                         % ", ".join(missing))
+
+
+def _main_bands(step_args, **fargs):
+    """``--latitude_bands``: this process is one rank of a torchrun job; it binds its GPU, sets up NCCL (the
+    engine's status exchange) and a gloo group (the host-side agreement) and runs the band pipeline over every
+    file."""
+    import torch
+    import torch.distributed as dist
+    from .parallel import bind_to_gpu_numa
+    local = int(os.environ["LOCAL_RANK"])
+    torch.cuda.set_device(local)
+    bind_to_gpu_numa(local)
+    dist.init_process_group("nccl", device_id=torch.device("cuda", local))
+    try:
+        return pgw_for_era5_files(step_args, band=Band(dist.group.WORLD, dist.new_group(backend="gloo")), **fargs)
+    finally:
+        dist.destroy_process_group()
 
 
 def main(argv=None):
@@ -451,8 +734,10 @@ def main(argv=None):
     last_era_step = datetime.strptime(args.last_era_step, '%Y%m%d%H')
     era_step_dts = np.arange(first_era_step, last_era_step + timedelta(hours=args.hour_inc_step),
                              timedelta(hours=args.hour_inc_step)).tolist()
+    if args.latitude_bands:
+        _check_band_args(args)
     Path(args.output_dir).mkdir(parents=True, exist_ok=True)
-    IMP = IterMP(njobs=args.n_par, run_async=True)
+    IMP = None if args.latitude_bands else IterMP(njobs=args.n_par, run_async=True)
     fargs = dict(delta_input_dir=args.delta_input_dir,
                  ignore_top_pressure_error=args.ignore_top_pressure_error, debug_mode=args.debug_mode)
     step_args = []
@@ -462,6 +747,8 @@ def main(argv=None):
         step_args.append(dict(inp_era_file_path=os.path.join(args.input_dir, name),
                               out_era_file_path=os.path.join(args.output_dir, name),
                               era_step_dt=era_step_dt))
+    if args.latitude_bands:
+        return _main_bands(step_args, **fargs)
     if args.debug_mode is None:
         # production mode: every worker (GPU) gets its share of the files and pipelines reading,
         # the CUDA pass and writing (the reference hands single files to its pool, :601-638)
