@@ -314,6 +314,11 @@ long long pgw_timestep_smem_bytes(const pgw_timestep_args *a);
  * PGW_FLAG_REF_DTYPES, and PGW_FLAG_LOCAL_PREF and PGW_FLAG_REINTERP on every grid: the TMA flavour handles a
  * scalar p_ref and iteration-invariant parked levels only) */
 int pgw_timestep_uses_tma(const pgw_timestep_args *a);
+/* The plan pgw_timestep() launches for these args: info[0] 1 for the TMA flavour, info[1] 1 if every layer the
+ * iteration can touch takes the ln series (the FAST instances; 0: the exact-log ones), info[2] the top level of
+ * the stash, info[3] the number of parked levels, info[4] the tensor-memory columns per CTA (0 for cp.async),
+ * info[5] 1 if the TMA flavour takes its L137 instance (137 levels, 56 parked).  PGW_OK or PGW_E_INVALID. */
+int pgw_timestep_plan_info(const pgw_timestep_args *a, int info[6]);
 /* Resources per CTA of the TMA flavour for nplev pressure nodes, nlev levels and np parked levels (even): the
  * tensor-memory columns it allocates and the bytes of dynamic shared memory it is launched with (padded to the
  * CTA's share of the SM's tensor memory).  Host arithmetic only; PGW_E_INVALID for arguments out of range. */

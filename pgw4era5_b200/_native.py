@@ -115,6 +115,7 @@ def _load():
         "pgw_time_mean_f32": (i, [vp, i, vp, ll, vp]),
         "pgw_timestep_smem_bytes": (ll, [C.POINTER(TimestepArgs)]),
         "pgw_timestep_uses_tma": (i, [C.POINTER(TimestepArgs)]),
+        "pgw_timestep_plan_info": (i, [C.POINTER(TimestepArgs), C.POINTER(C.c_int * 6)]),
         "pgw_column_tma_layout": (i, [i, i, i, C.POINTER(C.c_int), C.POINTER(C.c_longlong)]),
         "pgw_timestep": (i, [C.POINTER(TimestepArgs), vp]),
         "pgw_timestep_finalize": (i, [C.POINTER(TimestepArgs), vp, vp]),
@@ -165,3 +166,13 @@ def check(rc, what):
     name = {PGW_E_INVALID: "invalid argument", PGW_E_LAUNCH: "CUDA error", PGW_E_SMEM:
             "shared memory"}.get(rc, "error %d" % rc)
     raise NativeError("%s: %s %s" % (what, name, msg))
+
+
+PLAN_KEYS = ("tma", "fast", "lst", "np", "tmem_cols", "l137")
+
+
+def plan_info(args):
+    """The column-kernel plan pgw_timestep() launches for ``args`` (pgw_timestep_plan_info), as a dict."""
+    info = (C.c_int * 6)()
+    check(lib.pgw_timestep_plan_info(C.byref(args), C.byref(info)), "pgw_timestep_plan_info")
+    return dict(zip(PLAN_KEYS, info))

@@ -373,6 +373,10 @@ struct pgw_column_plan {
 // pgw_column_tma.cu
 bool pgw_tma_eligible(const pgw_timestep_args *a, int lst_generic, int *lst_tma, size_t *smem);
 int pgw_launch_column_tma(const pgw_timestep_args *a, const pgw_column_plan &plan, cudaStream_t st);
+// the TMA launch takes the instance compiled for 137 levels and 56 parked ones
+bool pgw_tma_l137(const pgw_timestep_args *a, const pgw_column_plan &plan);
+// tensor-memory columns per CTA of the TMA flavour for np parked levels
+int pgw_tma_tmem_cols(int np);
 // Opt a kernel in to `smem` bytes of dynamic shared memory on the CURRENT device.  The attribute is per device
 // and per kernel; `slot` (0..15) names the kernel variant in a per-device table of what has been configured.
 int pgw_ensure_smem(const void *kernel, int slot, size_t smem, int np);

@@ -862,6 +862,12 @@ bool pgw_tma_eligible(const pgw_timestep_args *a, int lst_generic, int *lst_tma,
     return true;
 }
 
+bool pgw_tma_l137(const pgw_timestep_args *a, const pgw_column_plan &plan) {
+    return a->nlev == 137 && plan.np == 56 && plan.lst == 137 - 56;
+}
+
+int pgw_tma_tmem_cols(int np) { return tmem_cols_tma(np); }
+
 int pgw_launch_column_tma(const pgw_timestep_args *a, const pgw_column_plan &plan, cudaStream_t st) {
     int rc;
     pgw::TmaParams tp;
@@ -873,7 +879,7 @@ int pgw_launch_column_tma(const pgw_timestep_args *a, const pgw_column_plan &pla
     }
     for (int l = 0; l < pgw::kTmaMaxLev; ++l)
         tp.m[l] = l < a->nlev ? make_float2((float)a->akm_host[l], (float)a->bkm_host[l]) : make_float2(0.f, 0.f);
-    const bool l137 = a->nlev == 137 && plan.np == 56 && plan.lst == 137 - 56;
+    const bool l137 = pgw_tma_l137(a, plan);
     auto kern = plan.fast ? (l137 ? pgw::pgw_column_tma_kernel<true, 137, 56> : pgw::pgw_column_tma_kernel<true, 0, 0>)
                           : (l137 ? pgw::pgw_column_tma_kernel<false, 137, 56> : pgw::pgw_column_tma_kernel<false, 0, 0>);
     if ((rc = pgw_ensure_smem((const void *)kern, 4 + (plan.fast ? 1 : 0) + (l137 ? 2 : 0), plan.smem, plan.np)) != PGW_OK)

@@ -1065,6 +1065,19 @@ int pgw_timestep_uses_tma(const pgw_timestep_args *a) {
     return plan_column(a).tma ? 1 : 0;
 }
 
+int pgw_timestep_plan_info(const pgw_timestep_args *a, int info[6]) {
+    int rc = validate(a);
+    if (rc != PGW_OK || !info) return PGW_E_INVALID;
+    const pgw_column_plan p = plan_column(a);
+    info[0] = p.tma ? 1 : 0;
+    info[1] = p.fast && !p.ref ? 1 : 0;           // PGW_FLAG_REF_DTYPES has one instance, the exact-log one
+    info[2] = p.lst;
+    info[3] = p.np;
+    info[4] = p.tma ? pgw_tma_tmem_cols(p.np) : 0;
+    info[5] = p.tma && pgw_tma_l137(a, p) ? 1 : 0;
+    return PGW_OK;
+}
+
 int pgw_timestep(const pgw_timestep_args *a, void *stream) {
     int rc = validate(a);
     if (rc != PGW_OK) return rc;
