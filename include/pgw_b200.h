@@ -27,11 +27,12 @@
 extern "C" {
 #endif
 
-#define PGW_B200_ABI_VERSION 9   /* 6: + pgw_timestep_status, pgw_timestep_run/_finish, PGW_FLAG_REF_DTYPES, first_k,
+#define PGW_B200_ABI_VERSION 10  /* 6: + pgw_timestep_status, pgw_timestep_run/_finish, PGW_FLAG_REF_DTYPES, first_k,
                                        pgw_band_pack/_unpack, pgw_band_exchange, pgw_regrid_bilinear_band_f32
                                     7: + PGW_FLAG_LOCAL_PREF and its args, PGW_ERR_PREF_FLOOR, first_k[4]
                                     8: + PGW_FLAG_REINTERP (no layout change)
-                                    9: + pgw_pack_d4_f32 */
+                                    9: + pgw_pack_d4_f32
+                                   10: + pgw_regrid_pack_d4_f32, PGW_REGRID_PACK_MAX_NX_S */
 
 /* host-side return codes */
 #define PGW_OK               0
@@ -476,6 +477,22 @@ int pgw_byteswap32(void *data, long long n, void *stream);
  * ---------------------------------------------------------------------- */
 int pgw_pack_d4_f32(const void *ta, const void *hur, const void *ua, const void *va, void *out, long long n,
                     int swap, void *stream);
+
+/* ------------------------------------------------------------------------
+ * Climatology on the GCM grid: one delta stamp of ta, hur, ua, va regridded to the ERA5 grid and packed in one
+ * pass, bit-identical to pgw_regrid_bilinear_band_f32 on each variable followed by pgw_pack_d4_f32.
+ *   src [4, nlev, ny_s, nx_s] (ta, hur, ua, va), polemean [4 * nlev, 2] (pgw_zonal_mean_f32 of src),
+ *   tables and target rows [jt_begin, jt_end) as for pgw_regrid_bilinear_band_f32,
+ *   dst float4 [nlev, jt_end - jt_begin, nx_t] (16-byte aligned).
+ * Source rows up to PGW_REGRID_PACK_MAX_NX_S columns run in the fused kernel and scratch may be NULL.  Wider
+ * ones are regridded variable by variable into scratch (16-byte aligned, 4 pieces of n = nlev * (jt_end -
+ * jt_begin) * nx_t floats, each rounded up to a multiple of 4) and then packed.
+ * ---------------------------------------------------------------------- */
+#define PGW_REGRID_PACK_MAX_NX_S 1536    /* the latitude-blended row of the four variables in 48 KB of shared memory */
+int pgw_regrid_pack_d4_f32(const float *src, float *dst, const float *polemean, int nlev, int ny_s, int nx_s,
+                           int ny_t, int nx_t, int jt_begin, int jt_end, const int *j0, const int *j1,
+                           const double *wy, const int *i0, const int *i1, const double *wx, float *scratch,
+                           void *stream);
 
 #ifdef __cplusplus
 }

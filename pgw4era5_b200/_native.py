@@ -36,6 +36,7 @@ FLAG_REINTERP = 8
 RUN_NO_FINALIZE = 1
 BAND_WORDS = 64 + 2 + 32 + 4
 INT32_MAX = 2 ** 31 - 1
+REGRID_PACK_MAX_NX_S = 1536     # PGW_REGRID_PACK_MAX_NX_S: wider GCM grids need the scratch of pgw_regrid_pack_d4_f32
 
 EXTRAP_MODES = {"off": 0, "linear": 1, "constant": 2, "nan": 3}
 
@@ -73,7 +74,7 @@ class TimestepStatus(C.Structure):
                 ("err", C.c_uint32), ("first_k", C.c_int32 * 4), ("poly_fallback", C.c_uint32)]
 
 
-ABI_VERSION = 9         # PGW_B200_ABI_VERSION of include/pgw_b200.h
+ABI_VERSION = 10        # PGW_B200_ABI_VERSION of include/pgw_b200.h
 
 
 class NativeError(RuntimeError):
@@ -128,6 +129,7 @@ def _load():
         "pgw_zonal_mean_f32": (i, [vp, vp, ll, i, i, vp]),
         "pgw_regrid_bilinear_f32": (i, [vp, vp, vp, ll, i, i, i, i, vp, vp, vp, vp, vp, vp, vp]),
         "pgw_regrid_bilinear_band_f32": (i, [vp, vp, vp, ll, i, i, i, i, i, i, vp, vp, vp, vp, vp, vp, vp]),
+        "pgw_regrid_pack_d4_f32": (i, [vp, vp, vp, i, i, i, i, i, i, i, vp, vp, vp, vp, vp, vp, vp, vp]),
         "pgw_smooth_harmonic_f32": (i, [vp, vp, i, ll, vp]),
         "pgw_surface_update": (i, [C.POINTER(TimestepArgs), vp]),
         "pgw_hybrid_pressure_f64": (i, [vp, vp, vp, vp, i, ll, vp]),

@@ -461,6 +461,52 @@ regrid_walk_kernel(const float *__restrict__ src, float *__restrict__ dst, const
 #undef PGW_WALK
 }
 
+// One delta stamp of ta, hur, ua, va from the GCM grid straight into the column kernel's node layout: dst is
+// float4 [K][jt_end - jt_begin][nx_t] = {ta, hur, ua, va}, what regrid_walk_kernel on each variable followed by
+// pack_d4_kernel writes.  A CTA takes one (level, target row) at a time: (1) the four variables' two bracketing
+// source rows are blended in latitude once per source column into shared memory (float64, functions.py:859),
+// (2) every thread produces target longitudes from that row (:892) and writes one 16-byte streaming store per
+// column.  Same expressions as regrid_kernel, hence bit-identical; the ~22 MB source of a stamp sits in L2, so
+// the kernel is bound by the store of the stamp, which it writes once instead of three times.
+constexpr int kRegridPackThreads = 256;
+
+__global__ void __launch_bounds__(kRegridPackThreads)
+regrid_pack_d4_kernel(const float *__restrict__ src, float4 *__restrict__ dst, const float *__restrict__ polemean,
+                      int nlev, int ny_s, int nx_s, int nx_t, int jt_begin, int jt_end, const int *__restrict__ j0,
+                      const int *__restrict__ j1, const double *__restrict__ wy, const int *__restrict__ i0,
+                      const int *__restrict__ i1, const double *__restrict__ wx) {
+    extern __shared__ double s_lat[];               // [4 variables][nx_s]: the row blended in latitude
+    const int nrow = jt_end - jt_begin;
+    const long long nitem = (long long)nlev * nrow;
+    const size_t var_stride = (size_t)nlev * ny_s * nx_s;
+    for (long long item = blockIdx.x; item < nitem; item += gridDim.x) {
+        const int k = (int)(item / nrow), r = (int)(item % nrow), jt = jt_begin + r;
+        const int ja = j0[jt], jb = j1[jt];
+        const double wj = wy[jt];
+        __syncthreads();                            // the previous item's longitude pass is done with s_lat
+        for (int idx = threadIdx.x; idx < 4 * nx_s; idx += blockDim.x) {
+            const int v = idx / nx_s, i = idx - v * nx_s;
+            const float *fld = src + v * var_stride + (size_t)k * ny_s * nx_s;
+            const float *pm = polemean + 2 * ((long long)v * nlev + k);
+            const double a0 = src_at(fld, pm, ja, i, nx_s), a1 = src_at(fld, pm, jb, i, nx_s);
+            s_lat[idx] = (a1 - a0) * wj + a0;       // latitude pass (functions.py:859)
+        }
+        __syncthreads();
+        float4 *o = dst + ((size_t)k * nrow + r) * (size_t)nx_t;
+        for (int it = threadIdx.x; it < nx_t; it += blockDim.x) {
+            const int ia = __ldg(i0 + it), ib = __ldg(i1 + it);
+            const double w = __ldg(wx + it);
+            float res[4];
+#pragma unroll
+            for (int v = 0; v < 4; ++v) {
+                const double a = s_lat[v * nx_s + ia], b = s_lat[v * nx_s + ib];
+                res[v] = (float)((b - a) * w + a);  // longitude pass (:892)
+            }
+            __stcs(o + it, make_float4(res[0], res[1], res[2], res[3]));
+        }
+    }
+}
+
 // harmonic_ac_analysis (functions.py:678-740): mean + harmonics 1..3 of an
 // nt-long series per grid point.  One thread per grid point, lanes = adjacent
 // points; cos/sin tables for the three harmonics are staged in shared memory.
@@ -656,6 +702,37 @@ int pgw_regrid_bilinear_f32(const float *src, float *dst, const float *polemean,
         regrid_kernel<1><<<(unsigned)g, 256, 0, (cudaStream_t)stream>>>(src, dst, polemean, nfield, ny_s, nx_s,
                                                                          ny_t, nx_t, j0, j1, wy, i0, i1, wx);
     return pgw_check_launch("regrid_kernel");
+}
+
+int pgw_regrid_pack_d4_f32(const float *src, float *dst, const float *polemean, int nlev, int ny_s, int nx_s,
+                           int ny_t, int nx_t, int jt_begin, int jt_end, const int *j0, const int *j1,
+                           const double *wy, const int *i0, const int *i1, const double *wx, float *scratch,
+                           void *stream) {
+    if (!src || !dst || !polemean || !j0 || !j1 || !wy || !i0 || !i1 || !wx) return PGW_E_INVALID;
+    if (nlev < 1 || ny_s < 1 || nx_s < 1 || ny_t < 1 || nx_t < 1) return PGW_E_INVALID;
+    if (jt_begin < 0 || jt_end > ny_t || jt_begin >= jt_end) return PGW_E_INVALID;
+    if ((reinterpret_cast<uintptr_t>(dst) & 15u) != 0) return PGW_E_INVALID;
+    const int nrow = jt_end - jt_begin;
+    if (nx_s <= PGW_REGRID_PACK_MAX_NX_S) {
+        const size_t smem = sizeof(double) * 4 * (size_t)nx_s;          // <= 48 KB: no opt-in
+        const long long nitem = (long long)nlev * nrow;
+        const long long g = nitem < 148LL * 8 ? nitem : 148LL * 8;
+        regrid_pack_d4_kernel<<<(unsigned)g, kRegridPackThreads, smem, (cudaStream_t)stream>>>(
+            src, reinterpret_cast<float4 *>(dst), polemean, nlev, ny_s, nx_s, nx_t, jt_begin, jt_end, j0, j1, wy, i0,
+            i1, wx);
+        return pgw_check_launch("regrid_pack_d4_kernel");
+    }
+    // wider source rows: each variable regridded into the scratch, then packed (the same expressions)
+    if (!scratch || (reinterpret_cast<uintptr_t>(scratch) & 15u) != 0) return PGW_E_INVALID;
+    const long long n = (long long)nlev * nrow * nx_t, piece = (n + 3) / 4 * 4;
+    const long long field = (long long)ny_s * nx_s;
+    int rc;
+    for (int v = 0; v < 4; ++v)
+        if ((rc = pgw_regrid_bilinear_band_f32(src + v * nlev * field, scratch + v * piece, polemean + 2LL * v * nlev,
+                                               nlev, ny_s, nx_s, ny_t, nx_t, jt_begin, jt_end, j0, j1, wy, i0, i1, wx,
+                                               stream)) != PGW_OK)
+            return rc;
+    return pgw_pack_d4_f32(scratch, scratch + piece, scratch + 2 * piece, scratch + 3 * piece, dst, n, 0, stream);
 }
 
 int pgw_smooth_harmonic_f32(const float *series, float *out, int nt, long long npoint, void *stream) {

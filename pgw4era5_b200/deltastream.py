@@ -81,23 +81,22 @@ def choose_slot(keys, ticks, busy):
 
 
 class _Ring:
-    """``slots`` device buffers of one stamp each, loaded from ``sources`` through one pinned staging buffer."""
+    """``slots`` device buffers of one stamp each (``words`` floats per variable, ``nvar`` = 4 packed variables or
+    1): which slot holds which stamp, eviction and the device-side waits for the slots' users.  A subclass fills a
+    slot: ``_stage`` on the host, then ``_fill`` on the set's copy stream, which must wait for ``_wait_uses`` before
+    it writes the slot."""
 
-    def __init__(self, owner, name, sources, keep, words, slots):
+    def __init__(self, owner, name, keep, words, nvar, slots):
         dev = owner.device
-        self.owner, self.name, self.sources, self.keep, self.n = owner, name, sources, keep, words
-        self.packed = len(sources) == 4
-        self.swap = sources[0].swap
-        self.stride = (words + 3) // 4 * 4                  # 16-byte aligned pieces: vector loads in the pack
-        self.host = torch.empty(len(sources) * self.stride, dtype=torch.float32, pin_memory=True)
-        self.host_free = torch.cuda.Event()
-        self.raw = torch.empty(4 * self.stride, device=dev, dtype=torch.float32) if self.packed else None
-        self.bufs = [torch.empty(words * (4 if self.packed else 1), device=dev, dtype=torch.float32)
-                     for _ in range(slots)]
+        self.owner, self.name, self.keep, self.n = owner, name, keep, words
+        self.bufs = [torch.empty(words * nvar, device=dev, dtype=torch.float32) for _ in range(slots)]
         self.keys, self.ticks = [None] * slots, [0] * slots
         self.ready = [torch.cuda.Event() for _ in range(slots)]
         self.uses = [{} for _ in range(slots)]              # stream -> last use event (a stream runs in order)
         self.pending, self.clock, self.loads = set(), 0, 0
+
+    def device_tensors(self):
+        return list(self.bufs)
 
     def acquire(self, i, other=None):
         """Slot of kept stamp ``i`` (-1: the last, the year wrap), loaded on a miss; the slot of kept stamp
@@ -117,36 +116,25 @@ class _Ring:
         torch.cuda.current_stream().wait_event(self.ready[s])
         return s
 
+    def _wait_uses(self, s, stream):
+        for e in self.uses[s].values():
+            stream.wait_event(e)
+
+    def _stage(self, rec):
+        """Host work of a load, before anything is queued on the copy stream."""
+
     def _load(self, s, i):
         rec = stamp_record(self.keep, i)
         timing = self.owner.load_events
         t0 = time.perf_counter()
-        self.host_free.synchronize()
-        for j, src in enumerate(self.sources):
-            src.read(rec, self.host[j * self.stride:j * self.stride + self.n])
+        self._stage(rec)
         t1 = time.perf_counter()
         cs = self.owner.copy_stream
         with torch.cuda.stream(cs):
             ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)] if timing is not None else None
             if ev:
                 ev[0].record(cs)
-            if not self.packed:
-                for e in self.uses[s].values():
-                    cs.wait_event(e)
-            dst = self.raw if self.packed else self.bufs[s]
-            dst.copy_(self.host[:dst.numel()], non_blocking=True)
-            self.host_free.record(cs)
-            if ev:
-                ev[1].record(cs)
-            st = C.c_void_p(cs.cuda_stream)
-            if self.packed:
-                for e in self.uses[s].values():
-                    cs.wait_event(e)
-                p = [C.c_void_p(self.raw.data_ptr() + 4 * j * self.stride) for j in range(4)]
-                N.check(N.lib.pgw_pack_d4_f32(*p, C.c_void_p(self.bufs[s].data_ptr()), self.n, self.swap, st),
-                        "pgw_pack_d4_f32")
-            elif self.swap:
-                N.check(N.lib.pgw_byteswap32(C.c_void_p(self.bufs[s].data_ptr()), self.n, st), "pgw_byteswap32")
+            self._fill(s, rec, cs, ev)
             if ev:
                 ev[2].record(cs)
             self.ready[s].record(cs)
@@ -155,6 +143,46 @@ class _Ring:
         self.loads += 1
         if ev:
             timing.append(dict(ring=self.name, fill_s=t1 - t0, events=ev))
+
+
+class _HostRing(_Ring):
+    """A ring loaded from ``sources`` through one pinned staging buffer: the host reads the stamp, the copy stream
+    uploads it and packs it into the slot (zg: uploads it into the slot)."""
+
+    def __init__(self, owner, name, sources, keep, words, slots):
+        super().__init__(owner, name, keep, words, len(sources), slots)
+        self.sources = sources
+        self.packed = len(sources) == 4
+        self.swap = sources[0].swap
+        self.stride = (words + 3) // 4 * 4                  # 16-byte aligned pieces: vector loads in the pack
+        self.host = torch.empty(len(sources) * self.stride, dtype=torch.float32, pin_memory=True)
+        self.host_free = torch.cuda.Event()
+        self.raw = torch.empty(4 * self.stride, device=owner.device, dtype=torch.float32) if self.packed else None
+
+    def device_tensors(self):
+        return self.bufs + ([self.raw] if self.raw is not None else [])
+
+    def _stage(self, rec):
+        self.host_free.synchronize()
+        for j, src in enumerate(self.sources):
+            src.read(rec, self.host[j * self.stride:j * self.stride + self.n])
+
+    def _fill(self, s, rec, cs, ev):
+        if not self.packed:
+            self._wait_uses(s, cs)
+        dst = self.raw if self.packed else self.bufs[s]
+        dst.copy_(self.host[:dst.numel()], non_blocking=True)
+        self.host_free.record(cs)
+        if ev:
+            ev[1].record(cs)
+        st = C.c_void_p(cs.cuda_stream)
+        if self.packed:
+            self._wait_uses(s, cs)
+            p = [C.c_void_p(self.raw.data_ptr() + 4 * j * self.stride) for j in range(4)]
+            N.check(N.lib.pgw_pack_d4_f32(*p, C.c_void_p(self.bufs[s].data_ptr()), self.n, self.swap, st),
+                    "pgw_pack_d4_f32")
+        elif self.swap:
+            N.check(N.lib.pgw_byteswap32(C.c_void_p(self.bufs[s].data_ptr()), self.n, st), "pgw_byteswap32")
 
 
 class StreamedDeltaSet(DeltaSetBase):
@@ -200,6 +228,21 @@ class StreamedDeltaSet(DeltaSetBase):
             if tuple(sources[name].shape[-2:]) != self.shape2d:
                 raise ValueError("%s delta is on a %s grid, the 2-D deltas on %s" % (name, sources[name].shape[-2:],
                                                                                      self.shape2d))
+        self._upload_2d(flat)
+        self.sources = sources
+        self.copy_stream = torch.cuda.Stream(device=self.device)
+        # set to [] to collect every load: the host fill time and three CUDA events on the copy stream (start; upload
+        # done, or the slot's users done for a regridded stamp; slot filled)
+        self.load_events = None
+        K, Kz = sources["ta"].shape[1], sources["zg"].shape[1]
+        self.rings = dict(d4=_HostRing(self, "d4", [sources[n] for n in VARS_PACKED], keeps["ta"], K * self.ncol,
+                                       slots),
+                          zg=_HostRing(self, "zg", [sources["zg"]], keeps["zg"], Kz * self.ncol, slots))
+        self.ts_clim = None
+        self.refresh_derived()
+
+    def _upload_2d(self, flat):
+        """The 2-D deltas (name -> [nt, ny, nx] tensor, 29 February dropped) into one device arena."""
         offs, total = {}, 0
         for name in VARS_2D:
             offs[name] = total
@@ -209,18 +252,10 @@ class StreamedDeltaSet(DeltaSetBase):
             v = self.arena[offs[name]:offs[name] + flat[name].numel()].view(flat[name].shape)
             v.copy_(flat.pop(name).to(self.device, torch.float32))
             self.vars[name]["data"] = v
-        self.sources = sources
-        self.copy_stream = torch.cuda.Stream(device=self.device)
-        self.load_events = None         # set to [] to collect the host fill time and CUDA events of every load
-        K, Kz = sources["ta"].shape[1], sources["zg"].shape[1]
-        self.rings = dict(d4=_Ring(self, "d4", [sources[n] for n in VARS_PACKED], keeps["ta"], K * self.ncol, slots),
-                          zg=_Ring(self, "zg", [sources["zg"]], keeps["zg"], Kz * self.ncol, slots))
-        self.ts_clim = None
-        self.refresh_derived()
 
     def device_bytes(self):
         """Device memory of the set: the 2-D arena, the ring slots and the packing buffer."""
-        ts = [self.arena] + [b for r in self.rings.values() for b in r.bufs + ([r.raw] if r.raw is not None else [])]
+        ts = [self.arena] + [t for r in self.rings.values() for t in r.device_tensors()]
         return sum(t.numel() * t.element_size() for t in ts)
 
     def hold(self, stream=None):

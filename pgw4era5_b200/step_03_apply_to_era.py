@@ -106,20 +106,44 @@ def _check_band_fits(whole, ny, device, max_resident_bytes, rows):
                          "%d ranks or more would fit" % fit if fit else "no number of ranks fits"))
 
 
-def get_engine(delta_input_dir, era_file, band=None):
+def load_gcm_grid_delta_set(delta_input_dir, era_file, device="cuda"):
+    """``GcmGridDeltaSet`` of the delta files of ``delta_input_dir`` still on the GCM grid (what step_02
+    regridding reads), regridded on the device to the grid of ``era_file`` (an ERA5 ``ncio.Dataset``).  Its
+    ``FR_LAND`` masks tos and siconc as the ``-e`` file of step_02 regridding does: the two must agree."""
+    from .gcmdeltas import GcmGridDeltaSet, read_gcm_deltas
+    land_fr = np.asarray(era_file[settings.var_name_map['sftlf']].data)[0]
+    return GcmGridDeltaSet(read_gcm_deltas(delta_input_dir), np.asarray(era_file[settings.LAT_ERA].data),
+                           np.asarray(era_file[settings.LON_ERA].data), land_fr, device=device)
+
+
+MSG_GCM_BANDS = "--gcm_grid_deltas does not run with --latitude_bands"
+MSG_GCM_INTERP_TIME = ("--gcm_grid_deltas does not run -D interpolate_time, which writes the time-interpolated "
+                       "deltas on the grid of the delta files: regrid them with step_02 first")
+
+
+def get_engine(delta_input_dir, era_file, band=None, gcm_grid_deltas=False):
     """One engine (and one resident copy of the climatology) per process and delta directory; with ``band``
-    (latitude-band mode, ``Band``) one per row range, holding the deltas of those rows only."""
+    (latitude-band mode, ``Band``) one per row range, holding the deltas of those rows only.  With
+    ``gcm_grid_deltas`` the delta files are on the GCM grid and regridded on the device to ``era_file``'s grid
+    (``load_gcm_grid_delta_set``)."""
     import torch
     from .engine import PGWEngine
+    if gcm_grid_deltas and band is not None:
+        raise ValueError(MSG_GCM_BANDS)
     ak = np.asarray(era_file['ak'].data)
     bk = np.asarray(era_file['bk'].data)
     key = (os.path.abspath(delta_input_dir), torch.cuda.current_device(), ak.tobytes(), bk.tobytes())
     if band is not None:
         key += (tuple(band.rows), band.exchange)
+    if gcm_grid_deltas:             # the deltas are regridded to this grid
+        key += ("gcm_grid", np.asarray(era_file[settings.LAT_ERA].data).tobytes(),
+                np.asarray(era_file[settings.LON_ERA].data).tobytes())
     eng = _ENGINES.get(key)
     if eng is None:
         device = torch.device("cuda", torch.cuda.current_device())
-        if band is None:
+        if gcm_grid_deltas:
+            ds = load_gcm_grid_delta_set(delta_input_dir, era_file, device)
+        elif band is None:
             ds = load_delta_set(delta_input_dir, device=device)
         else:
             # a band that does not fit, or a delta file one rank cannot read, must stop every rank before the
@@ -140,14 +164,17 @@ def get_engine(delta_input_dir, era_file, band=None):
 
 
 def pgw_for_era5(inp_era_file_path, out_era_file_path, delta_input_dir, era_step_dt,
-                 ignore_top_pressure_error, debug_mode=None):
-    """Same signature as the reference's pgw_for_era5 (step_03_apply_to_era.py:44-47)."""
+                 ignore_top_pressure_error, debug_mode=None, gcm_grid_deltas=False):
+    """Same signature as the reference's pgw_for_era5 (step_03_apply_to_era.py:44-47), plus ``gcm_grid_deltas``
+    (``get_engine``)."""
     import torch
     vmap = settings.var_name_map
+    if gcm_grid_deltas and debug_mode == 'interpolate_time':
+        raise ValueError(MSG_GCM_INTERP_TIME)
     if settings.i_debug >= 0:
         print('Start working on input file {}'.format(inp_era_file_path))
     era_file = ncio.open_dataset(inp_era_file_path, decode_cf=False)
-    eng = get_engine(delta_input_dir, era_file)
+    eng = get_engine(delta_input_dir, era_file, gcm_grid_deltas=gcm_grid_deltas)
     names = dict(PS=vmap['ps'], FIS=vmap['zgs'], FR_LAND=vmap['sftlf'], FR_SEA_ICE=vmap['sic'],
                  T_SKIN=vmap['ts'], T_SO=vmap['st'], T=vmap['ta'], QV=vmap['hus'], U=vmap['ua'], V=vmap['va'])
     era = {k: torch.from_numpy(np.ascontiguousarray(era_file[v].data, dtype=np.float32))
@@ -429,7 +456,8 @@ def _band_start(steps, names, band):
     return first, grid, tuple(rows)
 
 
-def pgw_for_era5_files(steps, delta_input_dir, ignore_top_pressure_error, debug_mode=None, band=None):
+def pgw_for_era5_files(steps, delta_input_dir, ignore_top_pressure_error, debug_mode=None, band=None,
+                       gcm_grid_deltas=False):
     """
     The production mode of ``pgw_for_era5`` for a LIST of files on one GPU, as a three-stage
     pipeline (SURVEY.md 8f rank 1): a reader thread decodes file i+1 into pinned host buffers and
@@ -448,11 +476,18 @@ def pgw_for_era5_files(steps, delta_input_dir, ignore_top_pressure_error, debug_
     before the start, before each file's submit and at the end, so a failure on one rank raises on all of them.
     Band mode runs whatever ``PGWEngine.submit`` runs (not the staged path, whose convergence test is per rank)
     on NetCDF-3 files; other settings and files raise ValueError before any GPU work.
+
+    ``gcm_grid_deltas``: the delta files are on the GCM grid and are regridded on the device to the grid of the
+    first file (``get_engine``); not with ``band`` nor with ``debug_mode = 'interpolate_time'`` (ValueError).
     """
     import queue
     import threading
     from concurrent.futures import ThreadPoolExecutor
     from .hostpipe import HostPipeline, IN_FIELDS
+    if gcm_grid_deltas and band is not None:
+        raise ValueError(MSG_GCM_BANDS)
+    if gcm_grid_deltas and debug_mode == 'interpolate_time':
+        raise ValueError(MSG_GCM_INTERP_TIME)
     if not steps:
         return []
     if band is not None:
@@ -461,7 +496,8 @@ def pgw_for_era5_files(steps, delta_input_dir, ignore_top_pressure_error, debug_
             raise ValueError(msg)
     elif debug_mode is not None or settings.i_reinterp or settings.p_ref_inp is None:
         return [pgw_for_era5(delta_input_dir=delta_input_dir,
-                             ignore_top_pressure_error=ignore_top_pressure_error, debug_mode=debug_mode, **st)
+                             ignore_top_pressure_error=ignore_top_pressure_error, debug_mode=debug_mode,
+                             gcm_grid_deltas=gcm_grid_deltas, **st)
                 for st in steps]
     vmap = settings.var_name_map
     names = _ERA_NAMES(vmap)
@@ -472,7 +508,7 @@ def pgw_for_era5_files(steps, delta_input_dir, ignore_top_pressure_error, debug_
     else:
         first, (ny, nx), rows = _band_start(steps, names, band)
         band = band._replace(rows=rows)
-    eng = get_engine(delta_input_dir, first, band)
+    eng = get_engine(delta_input_dir, first, band, gcm_grid_deltas=gcm_grid_deltas)
     pipe = HostPipeline(eng, rows[1] - rows[0], nx)
     n_in_buf, n_out_buf = 3, 4
     free_in, free_out = queue.Queue(), queue.Queue()
@@ -633,9 +669,11 @@ def _run_file_group(steps, **fargs):
 
 
 def debug_interpolate_time(inp_era_file_path, out_era_file_path, delta_input_dir, era_step_dt,
-                           ignore_top_pressure_error, debug_mode=None):
+                           ignore_top_pressure_error, debug_mode=None, gcm_grid_deltas=False):
     """step_03_apply_to_era.py:387-414: write the deltas interpolated in time only."""
     from . import functions as F
+    if gcm_grid_deltas:
+        raise ValueError(MSG_GCM_INTERP_TIME)
     era_file = ncio.open_dataset(inp_era_file_path, decode_cf=False)
     for var_name in ['tos', 'tas', 'hurs', 'ps', 'ta', 'hur', 'ua', 'va', 'zg']:
         print(var_name)
@@ -687,6 +725,11 @@ def build_parser():
                         help='Run under torchrun, one rank per GPU: every rank reads, computes and writes its own '
                              'latitude rows of each file, holding only those rows of the climate deltas '
                              '(NetCDF-3 ERA5 files; not in the reference).')
+    parser.add_argument('--gcm_grid_deltas', action='store_true',
+                        help='The delta files in -d are still on the GCM grid (the input of step_02 regridding, '
+                             'normally the output of step_02 smoothing): regrid them on the GPU as step_02 '
+                             'regridding would, to the grid of the first ERA5 file, whose FR_LAND masks tos and '
+                             'siconc.  Not with --latitude_bands nor -D interpolate_time (not in the reference).')
     return parser
 
 
@@ -734,12 +777,18 @@ def main(argv=None):
     last_era_step = datetime.strptime(args.last_era_step, '%Y%m%d%H')
     era_step_dts = np.arange(first_era_step, last_era_step + timedelta(hours=args.hour_inc_step),
                              timedelta(hours=args.hour_inc_step)).tolist()
+    if args.gcm_grid_deltas and args.latitude_bands:
+        raise ValueError(MSG_GCM_BANDS)
+    if args.gcm_grid_deltas and args.debug_mode == 'interpolate_time':
+        raise ValueError(MSG_GCM_INTERP_TIME)
     if args.latitude_bands:
         _check_band_args(args)
     Path(args.output_dir).mkdir(parents=True, exist_ok=True)
     IMP = None if args.latitude_bands else IterMP(njobs=args.n_par, run_async=True)
     fargs = dict(delta_input_dir=args.delta_input_dir,
                  ignore_top_pressure_error=args.ignore_top_pressure_error, debug_mode=args.debug_mode)
+    if args.gcm_grid_deltas:
+        fargs["gcm_grid_deltas"] = True
     step_args = []
     for era_step_dt in era_step_dts:
         print(era_step_dt)
